@@ -140,7 +140,6 @@ _EXPORTS = {
     "espm_h_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_finish": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_apply": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
-    "espm_h_scalars": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_reduce": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_finish": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),

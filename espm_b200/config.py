@@ -10,20 +10,14 @@ x_storage : "auto" | "dense" | "uint8" | "uint16"
     Storage of X on the device.  "auto" keeps count data (integers below 256 / 65536, fp32 arithmetic, nothing for
     remove_zeros_lines / normalize to patch) as uint8 / uint16 and streams 4x / 2x fewer bytes per pass; "dense" always
     stores the uploaded floating-point values (what BASELINE.json's fp32 / fp64 roofline figures are quoted on).
-native_loop : bool
-    Issue the launches of the iterations from native code (espm_run_iterations) instead of one ctypes call per kernel.
-speculate : bool
-    In the loop with stop tests, enqueue iteration t+1 before the host has looked at the scalars of iteration t (and
-    roll it back when a stop test fires).  Both switches exist for A/B measurements and debugging.
 speculate_h : bool
     simplex_H: espm_h_finish applies the lock-step bisection count of the previous H update right after its trace and
-    espm_h_apply only confirms it (and redoes the replay when the count changed).  Results are identical either way.
+    espm_h_apply only confirms it (and redoes the replay when the count changed).  Results are identical either way;
+    the tests compare the two bit for bit.
 """
 import os as _os
 
 distributed = "auto"
-native_loop = _os.environ.get("ESPM_B200_NATIVE_LOOP", "1") != "0"
-speculate = _os.environ.get("ESPM_B200_SPECULATE", "1") != "0"
 speculate_h = _os.environ.get("ESPM_B200_SPECULATE_H", "1") != "0"
 x_storage = "auto"
 device_init = True

@@ -88,12 +88,6 @@ static int check_state(const espm_state* st) {
     return ESPM_OK;
 }
 
-#ifndef ESPM_GWRES_DEFAULT
-#define ESPM_GWRES_DEFAULT 0
-#endif
-#ifndef ESPM_L2PIN_MB_DEFAULT
-#define ESPM_L2PIN_MB_DEFAULT 0
-#endif
 static XPassArgs make_args(const espm_state* st, bool w_pass) {
     XPassArgs a;
     memset(&a, 0, sizeof(a));
@@ -122,30 +116,6 @@ static XPassArgs make_args(const espm_state* st, bool w_pass) {
     a.y_shift = (!w_pass && (st->flags & ESPM_FLAG_HQ)) ? st->log_shift : 0.0;
     a.n = st->n;
     a.p_loc = st->p_loc;
-    if (!w_pass) {
-        // resident GW: the planner appended the region to the H pass's shared memory (espm_plan)
-        XPassSizes z;
-        if (sizes_of(st, 1, &z) == ESPM_OK) {
-            const int csz = st->c_dtype == ESPM_F64 ? 8 : 4;
-            const int gw_al = (st->n_pad * st->kp * csz + 127) / 128 * 128;
-            const int extra = st->h_smem - (z.fixed + st->h_depth * z.h_stride + z.h_tail);
-            a.gw_res_off = (extra >= gw_al && extra > 0) ? st->h_smem - gw_al : 0;
-        }
-    }
-    {
-        // L2-resident part of X (see XPassArgs::pin_tiles): ESPM_B200_L2PIN_MB megabytes of the tile-major image
-        static int pin_mb = -1;
-        if (pin_mb < 0) {
-            const char* e = getenv("ESPM_B200_L2PIN_MB");
-            pin_mb = e ? atoi(e) : ESPM_L2PIN_MB_DEFAULT;
-            if (pin_mb < 0) pin_mb = 0;
-        }
-        const size_t item = st->x_dtype == ESPM_F64 ? 8 : st->x_dtype == ESPM_F32 ? 4 : st->x_dtype == ESPM_U16 ? 2 : 1;
-        const size_t tile_bytes = (size_t)st->n_pad * TILE_PX * item;
-        long long t = tile_bytes ? (long long)(((size_t)pin_mb << 20) / tile_bytes) : 0;
-        if (t > st->n_tiles) t = st->n_tiles;
-        a.pin_tiles = (int)t;
-    }
     return a;
 }
 
@@ -234,35 +204,12 @@ int espm_plan(espm_state* st) {
     // ---- H pass ----
     int depth = (budget_for(z.h_occ) - z.fixed - z.h_tail) / z.h_stride;
     if (depth > 8) depth = 8;
-    if (const char* e = getenv("ESPM_B200_HDEPTH")) {
-        const int d = atoi(e);
-        if (d >= 2 && d < depth) depth = d;
-    }
     if (depth < 2) {
         set_error("shared memory budget too small for the H pass (kp=%d)", st->kp);
         return ESPM_ERR_UNSUPPORTED;
     }
-    // GW resident in the H pass's shared memory (XPassArgs::gw_res_off) when all of it fits beside a ring of >= 3 stages
-    int gw_extra = 0;
-    {
-        static int on = -1;
-        if (on < 0) {
-            const char* e = getenv("ESPM_B200_GWRES");
-            on = e ? (atoi(e) != 0) : ESPM_GWRES_DEFAULT;
-        }
-        const int csz = st->c_dtype == ESPM_F64 ? 8 : 4;
-        const int gw_al = (st->n_pad * st->kp * csz + 127) / 128 * 128;
-        if (on && gw_al <= 40 * 1024) {
-            int d2 = (budget_for(z.h_occ) - z.fixed - z.h_tail - gw_al) / z.h_stride;
-            if (d2 > 8) d2 = 8;
-            if (d2 >= 3) {
-                if (d2 < depth) depth = d2;
-                gw_extra = gw_al;
-            }
-        }
-    }
     st->h_depth = depth;
-    st->h_smem = z.fixed + depth * z.h_stride + z.h_tail + gw_extra;
+    st->h_smem = z.fixed + depth * z.h_stride + z.h_tail;
     int occ = 0;
     {
         XPassLaunch l{XPASS_H, st->kp, 1, 1, st->h_smem, XMODE_KL};
@@ -292,10 +239,6 @@ int espm_plan(espm_state* st) {
             }
             if (eff >= 0.95) break;
         }
-        if (const char* e = getenv("ESPM_B200_HSPLIT")) {     // experiments
-            const int v = atoi(e);
-            if (v >= 1 && v <= NS) best = v;
-        }
         st->h_nsplit = best;
         const long long items = (long long)st->n_tiles * best;
         st->h_grid = (int)(items < cap_h ? items : cap_h);
@@ -308,13 +251,8 @@ int espm_plan(espm_state* st) {
         // Measured on B200 (C3 f32, profiles/r01f_summary.md): the W pass is FASTER with a shallow ring -- 6 stages
         // 0.347 ms, 5: 0.340, 4: 0.323, 3: 0.316, 2: 0.344.  Consecutive units of a CTA are 1 MiB apart in Xt (same
         // channel block, next tile), so every stage in flight opens another DRAM page; three stages per CTA keep the
-        // HBM queues short enough for the 592 concurrent streams.  ESPM_B200_WDEPTH overrides (experiments).
-        int wcap = 3;
-        if (const char* e = getenv("ESPM_B200_WDEPTH")) {
-            const int d = atoi(e);
-            if (d >= 2) wcap = d;
-        }
-        if (wdepth > wcap) wdepth = wcap;
+        // HBM queues short enough for the 592 concurrent streams.
+        if (wdepth > 3) wdepth = 3;
         if (wdepth < 2) {
             set_error("shared memory budget too small for the W pass (kp=%d)", st->kp);
             return ESPM_ERR_UNSUPPORTED;
@@ -440,7 +378,6 @@ int espm_gw_prepare(const espm_state* st, void* stream) { return small(OP_GW_PRE
 int espm_h_stats(const espm_state* st, void* stream) { return small(OP_H_STATS, st, stream); }
 int espm_h_finish(const espm_state* st, void* stream) { return small(OP_H_FINISH, st, stream); }
 int espm_h_apply(const espm_state* st, void* stream) { return small(OP_H_APPLY, st, stream); }
-int espm_h_scalars(const espm_state* st, void* stream) { return small(OP_H_SCALARS, st, stream); }
 int espm_w_reduce(const espm_state* st, void* stream) { return small(OP_W_REDUCE, st, stream); }
 int espm_w_finish(const espm_state* st, void* stream) { return small(OP_W_FINISH, st, stream); }
 

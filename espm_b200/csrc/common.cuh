@@ -106,15 +106,11 @@ inline cudaError_t launch_pdl(void (*kern)(KArgs...), dim3 grid, dim3 block, siz
     cfg.blockDim = block;
     cfg.dynamicSmemBytes = smem;
     cfg.stream = s;
-    static const bool enabled = [] {   // ESPM_B200_PDL=0 restores plain stream-ordered launches (A/B measurements)
-        const char* e = getenv("ESPM_B200_PDL");
-        return !(e && e[0] == '0');
-    }();
     cudaLaunchAttribute attr[1];
     attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
     attr[0].val.programmaticStreamSerializationAllowed = 1;
     cfg.attrs = attr;
-    cfg.numAttrs = enabled ? 1 : 0;
+    cfg.numAttrs = 1;
     return cudaLaunchKernelEx(&cfg, kern, std::forward<Args>(args)...);
 }
 

@@ -1066,7 +1066,7 @@ __global__ void __launch_bounds__(PX_THREADS, OCC) h_finish_kernel(const espm_st
         block_reduce_vals<NV>(vals, px_part_nsum(KP), st.px_part + (size_t)blockIdx.x * NV);
     }
     merge_mask(bits, err, (simplex && !(st.flags & ESPM_FLAG_EVAL_ONLY)) ? st.bisect_mask : nullptr, st.dev_flags);
-    // The last CTA to finish folds every partial into the scalar record (what espm_h_scalars does),
+    // The last CTA to finish folds every partial into the scalar record (h_scalars_block),
     // in a fixed order that does not depend on which CTA that is.
     __shared__ bool is_last;
     __threadfence();
@@ -1271,7 +1271,8 @@ __global__ void __launch_bounds__(256) hstats_reduce_kernel(const espm_state st)
 }
 
 // ------------------------------------------------------------------------------------------------
-// h_scalars: loss parts of the current iterate + rel_H + bisection count into the scalar record
+// h_scalars_block (last CTA of h_finish): loss parts of the current iterate + rel_H + bisection count into the
+// scalar record
 // ------------------------------------------------------------------------------------------------
 // `share` (optional): this rank's slot of its OWN record inbox (pixel-sharded fits; host memory every rank's process has
 // mapped): the additive / max / OR fields of the record that are per-shard quantities.  Written together with the record
@@ -1337,11 +1338,6 @@ __device__ __forceinline__ void h_scalars_block(const espm_state& st, double* sh
         *reinterpret_cast<volatile double*>(rec + ESPM_S_STAMP) = st.rec_stamp;
         if (share) *reinterpret_cast<volatile double*>(share + 7) = st.rec_stamp;
     }
-}
-
-template <typename TC>
-__global__ void __launch_bounds__(256) h_scalars_kernel(const espm_state st) {
-    h_scalars_block<TC>(st, nullptr);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -8,7 +8,6 @@ enum SmallOp {
     OP_H_FINISH = 0,
     OP_H_APPLY,
     OP_H_STATS,
-    OP_H_SCALARS,
     OP_W_REDUCE,
     OP_W_FINISH,
     OP_GW_PREPARE,
@@ -63,9 +62,6 @@ static int small_launch_t(int op, const espm_state* st, cudaStream_t s) {
             ESPM_KP_SWITCH(kp, (h_stats_kernel<TC, KP><<<st->px_blocks, PX_THREADS, 0, s>>>(*st)));
             ESPM_KP_SWITCH(kp, (hstats_reduce_kernel<TC, KP><<<1, 256, 0, s>>>(*st)));
             break;
-        case OP_H_SCALARS:
-            h_scalars_kernel<TC><<<1, 256, 0, s>>>(*st);
-            break;
         case OP_W_REDUCE: {
             const size_t total = (size_t)st->n_pad * st->kp;
             const int blocks = (int)((total + 255) / 256) + 1;
@@ -79,23 +75,19 @@ static int small_launch_t(int op, const espm_state* st, cudaStream_t s) {
             const void* fn = nullptr;
             ESPM_KP_SWITCH(kp, (fn = (const void*)w_finish_kernel<TC, KP>));
             // cooperative (grid barriers) AND programmatic dependent launch: the CTAs become resident while the W
-            // pass drains and wait in griddepcontrol.wait (ESPM_B200_PDL=0: plain stream order)
+            // pass drains and wait in griddepcontrol.wait
             cudaLaunchConfig_t cfg = {};
             cfg.gridDim = dim3(W_COOP_BLOCKS);
             cfg.blockDim = dim3(W_COOP_THREADS);
             cfg.dynamicSmemBytes = 0;
             cfg.stream = s;
-            static const bool pdl = [] {
-                const char* e = getenv("ESPM_B200_PDL");
-                return !(e && e[0] == '0');
-            }();
             cudaLaunchAttribute attr[2];
             attr[0].id = cudaLaunchAttributeCooperative;
             attr[0].val.cooperative = 1;
             attr[1].id = cudaLaunchAttributeProgrammaticStreamSerialization;
             attr[1].val.programmaticStreamSerializationAllowed = 1;
             cfg.attrs = attr;
-            cfg.numAttrs = pdl ? 2 : 1;
+            cfg.numAttrs = 2;
             ESPM_CUDA_CHECK(cudaLaunchKernelExC(&cfg, fn, args));
             break;
         }

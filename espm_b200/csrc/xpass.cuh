@@ -35,10 +35,6 @@ struct XPassArgs {
     double log_shift;
     double y_shift;      // H pass: ratio = x / (y + y_shift); log_shift for algo="l2_surrogate" (updates.py:280), else 0
     int n, p_loc;        // real channel / pixel counts (the Frobenius loss masks the padding)
-    int gw_res_off;      // H pass, non-SAFE instances: byte offset in shared memory where the CTA keeps ALL rows of GW for the
-                         // whole pass (0: the GW rows of a stage travel with it, a second bulk copy per stage)
-    int pin_tiles;       // X of the last pin_tiles tiles is fetched with the L2 evict_last policy by BOTH passes: that part
-                         // of the image stays in the 126 MB L2 from pass to pass and is not read from HBM again
 };
 
 // MODE of the X passes (template parameter):
@@ -48,10 +44,6 @@ struct XPassArgs {
 //   XMODE_KL_FROB H pass only: KL ratio sums, Frobenius loss (algo="l2_surrogate" with l2=True: the H step is
 //                 updates.py:263-301, the loss is 0.5 Frobenius_loss, base.py:197-198)
 constexpr int XMODE_KL = 0, XMODE_FROB = 1, XMODE_KL_FROB = 2;
-
-#ifndef ESPM_H_OCC_F64
-#define ESPM_H_OCC_F64 2
-#endif
 
 template <typename TX, typename TC, int KP, bool SAFE>
 struct XPassSmem {
@@ -75,8 +67,6 @@ struct XPassSmem {
     static constexpr bool ACC_REG = ACC_WORDS <= 64;
     // CTAs per SM the kernels are compiled for (register budget: 96 regs/thread at 2, 168 at 1)
     static constexpr int OCC_BASE = (KP * (int)sizeof(TC) <= 32) ? 2 : 1;
-    // fp64 H pass: ESPM_H_OCC_F64 = 1 trades half the warps for twice the registers (more independent DP chains per warp)
-    static constexpr int H_OCC = (OCC_BASE == 2 && sizeof(TC) == 8) ? ESPM_H_OCC_F64 : OCC_BASE;
     static constexpr int W_REGS_EST = (ACC_REG ? ACC_WORDS : KP * (int)sizeof(TC) / 4 * (FAST32 ? 2 : 1)) +
                                       KP * G::PPL * (int)sizeof(TC) / 4 + 36;
     static constexpr int W_OCC = (OCC_BASE == 2 && W_REGS_EST <= 110) ? 2 : 1;
@@ -232,7 +222,7 @@ struct Ring {
 // H pass
 // ------------------------------------------------------------------------------------------------
 template <typename TX, typename TC, int KP, bool SAFE, int MODE = XMODE_KL>
-__global__ void __launch_bounds__(XPASS_THREADS, (XPassSmem<TX, TC, KP, SAFE>::H_OCC))
+__global__ void __launch_bounds__(XPASS_THREADS, (XPassSmem<TX, TC, KP, SAFE>::OCC_BASE))
 h_pass_kernel(const XPassArgs a) {
     using G = PassGeom<TX, TC>;
     using S = XPassSmem<TX, TC, KP, SAFE>;
@@ -253,16 +243,6 @@ h_pass_kernel(const XPassArgs a) {
     pdl_wait();
     pdl_trigger();
     if (blockIdx.x == 0 && threadIdx.x < 4 && a.bisect_mask) a.bisect_mask[threadIdx.x] = 0u;
-    // GW resident in shared memory for the whole pass (n_pad x KP values, 32 KiB at C3): one bulk copy per stage
-    // instead of two, and the 512 B of GW rows per stage are not fetched from L2 131072 times per pass
-    const bool gw_res = !SAFE && a.gw_res_off != 0;
-    const unsigned char* gwres = smem + a.gw_res_off;
-    if (gw_res) {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(a.GW);
-        uint32_t* dst = reinterpret_cast<uint32_t*>(smem + a.gw_res_off);
-        const int words = a.n_pad * KP * (int)sizeof(TC) / 4;
-        for (int i = threadIdx.x; i < words; i += XPASS_THREADS) dst[i] = src[i];
-    }
     __syncthreads();
 
     const int n_items = a.n_tiles * a.nsplit;
@@ -273,7 +253,6 @@ h_pass_kernel(const XPassArgs a) {
         if (lane == 0) {
             const uint64_t pol_x = l2_policy_evict_first();
             const uint64_t pol_gw = l2_policy_evict_last();
-            const int pin0 = a.n_tiles - a.pin_tiles;
             const bool dual = SAFE && a.dual;
             typename Ring<S::H_STRIDE>::Pos pos{0, 0u};
             for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
@@ -283,10 +262,9 @@ h_pass_kernel(const XPassArgs a) {
                     ring.acquire(pos);
                     const int slot = pos.slot;
                     unsigned char* sp = ring.stage(slot);
-                    mbar_expect_tx(&ring.full[slot], S::X_BYTES + (gw_res ? 0 : S::GW_BYTES * (dual ? 2 : 1)));
+                    mbar_expect_tx(&ring.full[slot], S::X_BYTES + S::GW_BYTES * (dual ? 2 : 1));
                     const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)st * G::CS) * TILE_PX;
-                    tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[slot], tile >= pin0 ? pol_gw : pol_x);
-                    if (gw_res) continue;
+                    tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[slot], pol_x);
                     const TC* gsrc = reinterpret_cast<const TC*>(a.GW) + (size_t)st * G::CS * KP;
                     tma_bulk_g2s(sp + S::X_BYTES, gsrc, S::GW_BYTES, &ring.full[slot], pol_gw);
                     if (dual) {
@@ -331,7 +309,7 @@ h_pass_kernel(const XPassArgs a) {
             for (int st = s0; st < s1; ++st, ring.next(pos)) {
                 ring.consumer_wait(pos);
                 const unsigned char* xs = ring.stage(pos.slot);
-                const unsigned char* gs = gw_res ? gwres + (size_t)st * G::CS * KP * sizeof(TC) : xs + S::X_BYTES;
+                const unsigned char* gs = xs + S::X_BYTES;
                 float2 xl2 = make_float2(0.f, 0.f);
 #pragma unroll
                 for (int ci = 0; ci < G::CPW; ++ci) {
@@ -378,7 +356,7 @@ h_pass_kernel(const XPassArgs a) {
             for (int st = s0; st < s1; ++st, ring.next(pos)) {
                 ring.consumer_wait(pos);
                 const unsigned char* xs = ring.stage(pos.slot);
-                const unsigned char* gs = gw_res ? gwres + (size_t)st * G::CS * KP * sizeof(TC) : xs + S::X_BYTES;
+                const unsigned char* gs = xs + S::X_BYTES;
                 const unsigned char* gcs = gs + S::GW_BYTES_AL;
                 TC xl = TC(0);
                 float zl = 0.f;
@@ -567,7 +545,6 @@ w_pass_kernel(const XPassArgs a) {
         if (lane == 0) {
             const uint64_t pol_x = l2_policy_evict_first();
             const uint64_t pol_h = l2_policy_evict_last();
-            const int pin0 = a.n_tiles - a.pin_tiles;
             const TC* Ht = reinterpret_cast<const TC*>(a.Ht);
             typename Ring<S::W_STRIDE>::Pos pos{0, 0u};
             int cb = cb0, tile = tile0;
@@ -576,7 +553,7 @@ w_pass_kernel(const XPassArgs a) {
                 unsigned char* sp = ring.stage(pos.slot);
                 mbar_expect_tx(&ring.full[pos.slot], S::X_BYTES + KP * S::HROW_BYTES);
                 const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)cb * G::CS) * TILE_PX;
-                tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[pos.slot], tile >= pin0 ? pol_h : pol_x);
+                tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[pos.slot], pol_x);
                 tma_bulk_g2s(sp + S::X_BYTES, Ht + (size_t)tile * KP * TILE_PX, KP * S::HROW_BYTES, &ring.full[pos.slot],
                              pol_h);
                 if (++tile == a.n_tiles) {

@@ -98,7 +98,7 @@ static void xpass_sizes_kp(int safe, XPassSizes* o) {
     o->fixed = S0::BAR_BYTES + S0::MISC_BYTES;
     o->cs = S0::G::CS;
     o->halves = S0::G::HALVES;
-    o->h_occ = S0::H_OCC < S1::H_OCC ? S0::H_OCC : S1::H_OCC;
+    o->h_occ = S0::OCC_BASE;
     o->w_occ = S0::W_OCC < S1::W_OCC ? S0::W_OCC : S1::W_OCC;
 }
 

@@ -6,7 +6,7 @@ kernels in order on torch's current stream and rotates the W / H / GW buffers be
 
 One iteration of the reference (base.py:316-324) maps to two phases here:
 
-  phase A ``evaluate(slot)``   h_pass -> h_finish -> h_scalars
+  phase A ``evaluate(slot)``   h_pass -> h_finish (its last CTA writes the scalar record)
         streams X once with (GW_cur, H_cur): ratio sums for the next H update AND every loss term of
         the current iterate (KL, log-reg, Laplacian), rel_H, written to the scalar record ``slot``.
   phase B ``advance(slot)``    [h_apply] -> w_pass -> w_reduce -> w_finish, then buffer rotation

@@ -412,7 +412,7 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
     def _run_batch(self, eng, max_iter):
         """no_stop_criterion and nothing to print: enqueue every iteration, read the scalars once."""
         eng.evaluate(0)
-        if eng.fast_loop and config.native_loop:
+        if eng.fast_loop:
             eng.run_iterations(1, max_iter)          # one call: the launches of every iteration are issued natively
         else:
             for it in range(1, max_iter + 1):
@@ -453,10 +453,9 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         self._eval_init = eval_init
         self._final_rec = rec
         eval_before = np.inf
-        speculate = (self.physics_model_ is None and not self._track and not self.linesearch and not eng.pg_ls
-                     and config.speculate)
+        speculate = self.physics_model_ is None and not self._track and not self.linesearch and not eng.pg_ls
         ahead = False                      # is iteration n_iter_ + 1 already enqueued?
-        native = eng.fast_loop and not self._track and config.native_loop
+        native = eng.fast_loop and not self._track
 
         def step(i):
             if native:

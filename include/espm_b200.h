@@ -105,7 +105,7 @@ typedef enum espm_status {
 #define ESPM_DEV_NONFINITE_W  (1u << 6)  /* (with ESPM_DEV_NONFINITE) the non-finite sums came from the W pass (updates.py:53-56) */
 #define ESPM_DEV_PEER_TIMEOUT (1u << 5)  /* a peer rank did not signal within ~1 s: results of this fit are invalid */
 
-/* layout of one scalar record (doubles), written by espm_h_scalars / espm_w_finish */
+/* layout of one scalar record (doubles), written by espm_h_finish / espm_w_finish */
 enum {
     ESPM_S_XLOGY = 0,     /* sum max(X,ls)*log(Y) of the iterate fed to the H pass (measures.py:503) */
     ESPM_S_SUMY = 1,      /* sum Y = colsum(max(GW,ls)) . rowsum(max(H,ls)) (measures.py:502) */
@@ -352,14 +352,11 @@ int espm_h_pass(const espm_state* st, void* stream);
  * regularisers of the CURRENT iterate (measures.py:548,577), rel_H (base.py:324), and either
  *   simplex_H: the bisection bracket and the lock-step trace mask (dicotomy.py:29-49, 138-171), or
  *   otherwise: H_next = max(num/den, ls) (+fixed_H) directly (updates.py:152-155).
+ * Its last CTA reduces the H-side partials into st->scalars (loss parts of the current iterate, rel_H, flags).
  */
 int espm_h_finish(const espm_state* st, void* stream);
 /* Replays exactly it* bisection iterations (first clear bit of bisect_mask) and writes H_next (and Ht). */
 int espm_h_apply(const espm_state* st, void* stream);
-/* Reduces the H-side partials into st->scalars (loss parts of the current iterate, rel_H, flags).
- * espm_h_finish already does this in its last CTA; the entry point remains for callers that changed
- * st->scalars in between. */
-int espm_h_scalars(const espm_state* st, void* stream);
 
 /* W pass (updates.py:38-59, re-associated as G^T (R H^T)): streams Xt once with H_next.
  *   s_part[s][c][k] = sum_{j in the tiles CTA (first_cta(c/cs)+s) owns} X[c][j]/(GW.H_next)[c][j] * H_next[k][j] */
