@@ -41,6 +41,7 @@ FLAG_EVAL_ONLY = 1 << 19
 FLAG_LS_PARTIAL = 1 << 20
 FLAG_NO_HSPEC = 1 << 21
 FLAG_TIMING = 1 << 22
+FLAG_H_ONLY = 1 << 23
 COOP_BLOCKS = 32
 
 # device error word

@@ -470,6 +470,11 @@ int espm_run_iterations(espm_state* st, espm_loop* lp, int32_t first_slot, int32
         set_error("espm_run_iterations: this fit needs host work between the launches (Gram matrices / line search)");
         return ESPM_ERR_UNSUPPORTED;
     }
+    const bool h_only = (st->flags & ESPM_FLAG_H_ONLY) != 0;
+    if (h_only && (st->flags & ESPM_FLAG_PEER)) {
+        set_error("espm_run_iterations: ESPM_FLAG_H_ONLY on a pixel shard needs the host to combine the H' statistics");
+        return ESPM_ERR_UNSUPPORTED;
+    }
     cudaStream_t s = (cudaStream_t)stream;
     lp->launches = 0;
     loop_bind(st, lp);
@@ -481,6 +486,29 @@ int espm_run_iterations(espm_state* st, espm_loop* lp, int32_t first_slot, int32
         if (st->flags & ESPM_FLAG_SIMPLEX_H) {
             if ((rc = espm_h_apply(st, stream))) return rc;
             ++lp->launches;
+        }
+        if (h_only) {
+            // W stays: the row statistics of H' that w_finish would fold come from h_stats; only H / hstats rotate
+            if ((rc = espm_h_stats(st, stream))) return rc;
+            lp->launches += 2;
+            const int hp = lp->ih[0], hc = lp->ih[1], hn = lp->ih[2];
+            lp->ih[0] = hc;
+            lp->ih[1] = hn;
+            lp->ih[2] = hp;
+            const int s0 = lp->ihs[0];
+            lp->ihs[0] = lp->ihs[1];
+            lp->ihs[1] = s0;
+            lp->have_prev = 1;
+            loop_bind(st, lp);
+            lp->stamp += 1.0;
+            st->rec_stamp = lp->stamp;
+            st->seq_m = ++lp->seq_m;
+            if (ev && ev[2]) ESPM_CUDA_CHECK(cudaEventRecord((cudaEvent_t)ev[2], s));
+            if ((rc = espm_h_pass(st, stream))) return rc;
+            if (ev && ev[3]) ESPM_CUDA_CHECK(cudaEventRecord((cudaEvent_t)ev[3], s));
+            if ((rc = espm_h_finish(st, stream))) return rc;
+            lp->launches += 2;
+            continue;
         }
         st->seq_s = ++lp->seq_s;
         if (ev && ev[0]) ESPM_CUDA_CHECK(cudaEventRecord((cudaEvent_t)ev[0], s));

@@ -14,7 +14,8 @@ One iteration of the reference (base.py:316-324) maps to two phases here:
         GW_next; rel_W goes to record ``slot`` (the record of the iterate being produced).
 
 So X is read exactly twice per iteration (SURVEY.md section 8d); the loss of iterate t rides the H pass
-of iteration t+1.
+of iteration t+1.  With ``h_only`` (W fixed, ``SmoothNMF.transform``) phase B is [h_apply] -> h_stats and X is read
+once per iteration.
 """
 import ctypes
 
@@ -60,7 +61,7 @@ class FitEngine:
                  simplex_H=False, simplex_W=True, simplex_rows=None, fixed_H=None, fixed_W=None,
                  x_scale=1.0, max_records=512, device=None, shard=None, c_dtype=None, clamp_init=True,
                  x_local=False, ingest=None, algo="log_surrogate", l2=False, l2_h=False, linesearch=False,
-                 gamma_pg=None):
+                 gamma_pg=None, h_only=False):
         """
         X : (n, p) array-like view (any strides; C order or the transposed hyperspy layout are
             uploaded without a host copy).  G : (n, m) array or None (identity).  W0 : (m, k), H0 : (k, p).
@@ -70,6 +71,9 @@ class FitEngine:
             negative checks, remove_zeros_lines (base.py:519-528), normalize (base.py:264-267) and
             const_KL_ (base.py:200-201).  Results: ``self.const_KL``, ``self.norm_factor``,
             ``self.n_zero_rows`` / ``self.n_zero_cols``.
+        h_only : W0 is held fixed and only H is iterated (``SmoothNMF.transform``, ESPM_FLAG_H_ONLY): ``advance`` runs
+            [h_apply] -> h_stats and rotates the H buffers only, so an iteration streams X once (the H pass).  Only
+            the multiplicative H steps (``log_surrogate`` / ``l2_surrogate``) with the KL loss.
         """
         self.lib = L.load()
         self.clamp_init = clamp_init
@@ -160,6 +164,12 @@ class FitEngine:
             flags |= L.FLAG_L2_H                 # Frobenius H step / gradient (updates.py:109-118, 330-332)
         if flags & (L.FLAG_BMD | L.FLAG_PG | L.FLAG_L2):
             flags &= ~L.FLAG_SIMPLEX_W           # those W branches have no simplex projection (updates.py:29-48)
+        self.h_only = bool(h_only)
+        if self.h_only:
+            if flags & (L.FLAG_BMD | L.FLAG_PG | L.FLAG_L2 | L.FLAG_L2_H) or linesearch or fixed_W is not None:
+                raise ValueError("h_only supports the log_surrogate / l2_surrogate H steps with the KL loss, "
+                                 "without linesearch or fixed_W")
+            flags |= L.FLAG_H_ONLY
         self.pg_ls = False
         if linesearch:
             if flags & L.FLAG_PG:
@@ -255,6 +265,7 @@ class FitEngine:
             st.flags |= L.FLAG_LS_PARTIAL        # the sums of the line search are combined over the ranks on the host
         self._eval_slot = 0
         self._pg_w_pending = None
+        self._w_after_eval = None
         if gamma_pg is not None:
             st.gamma_h, st.gamma_w = float(gamma_pg[0]), float(gamma_pg[1])
         self.dev_flags = torch.zeros(8, dtype=torch.int32, device=dev)
@@ -591,7 +602,10 @@ class FitEngine:
         ls = self.st.log_shift
         wc, wn = self.iw
         W = torch.as_tensor(np.ascontiguousarray(W0), dtype=self.cdt).to(self.device)
-        Hs = torch.as_tensor(np.ascontiguousarray(H0[:, self.j0:self.j1]), dtype=self.cdt).to(self.device)
+        if isinstance(H0, torch.Tensor):         # e.g. the initial H computed on the device (init_device.py)
+            Hs = H0[:, self.j0:self.j1].to(self.device, self.cdt)
+        else:
+            Hs = torch.as_tensor(np.ascontiguousarray(H0[:, self.j0:self.j1]), dtype=self.cdt).to(self.device)
         if self.clamp_init:
             W, Hs = W.clamp_min(ls), Hs.clamp_min(ls)
         self.Wbuf[wn].copy_(W)
@@ -640,11 +654,31 @@ class FitEngine:
             L.check(self.lib.espm_gram(ctypes.byref(self.st), 0, self.stream))   # (G W)^T (G W), updates.py:115
         self._call(self.lib.espm_h_pass, "h_pass")
         self._call(self.lib.espm_h_finish, "h_finish")      # its last CTA also writes the scalar record
+        if self._w_after_eval is not None:
+            W, self._w_after_eval = self._w_after_eval, None
+            self._load_W(W)
+
+    def set_W_after_eval(self, W):
+        """H-only mode: the reference clamps W0 to log_shift (updates.py:220-221) but its fixed_W overwrites W with the
+        UNCLAMPED matrix in the first update (updates.py:75-76).  The evaluation of iterate 0 uses the clamped W given at
+        construction; ``W`` (unclamped) replaces it right after that evaluation is enqueued."""
+        self._w_after_eval = W
+
+    def _load_W(self, W):
+        """W_cur <- W as given (no clamp), GW / gwstats recomputed; stream-ordered after what is already enqueued."""
+        wc, wn = self.iw
+        self.Wbuf[wn].copy_(torch.as_tensor(np.ascontiguousarray(W), dtype=self.cdt).to(self.device))
+        self._set_record(self.max_records - 1)
+        self._call(self.lib.espm_gw_prepare)
+        self.iw = [wn, wc]
+        self._bind()
 
     def advance(self, slot):
         """Phase B: (W_cur, H_cur) -> (W_next, H_next), rotate.  rel_W etc. go to record ``slot``."""
         st = self.st
         self._set_record(slot)
+        if self.h_only:
+            return self._advance_h(st)
         if st.flags & L.FLAG_SIMPLEX_H:
             if self.shard is not None and not self.peer:
                 self.shard.gather_masks(self.mask)
@@ -679,13 +713,32 @@ class FitEngine:
         self.have_prev = True
         self._bind()
 
+    def _advance_h(self, st):
+        """Phase B with W fixed: H_cur -> H_next and its row statistics, then only the H buffers rotate (rel_W of the
+        record stays 0).  Sharded: the masks / halos as in ``advance`` and the H' statistics combined over the ranks."""
+        if st.flags & L.FLAG_SIMPLEX_H:
+            if self.shard is not None and not self.peer:
+                self.shard.gather_masks(self.mask)
+            self._call(self.lib.espm_h_apply, "h_apply")
+        if not self.peer:
+            self._exchange_halo(self.ih[2])
+        self._call(self.lib.espm_h_stats, "h_stats")
+        self.n_launches += 1                                 # espm_h_stats is two kernels
+        self._sync_hstats()
+        hp, hc, hn = self.ih
+        self.ih = [hc, hn, hp]
+        self.ihs = [self.ihs[1], self.ihs[0]]
+        self.have_prev = True
+        self._bind()
+
     # ------------------------------------------------------------------ the loop in native code
     @property
     def fast_loop(self):
-        """Can ``run_iterations`` be used?  Not when an iteration needs host work between its launches."""
+        """Can ``run_iterations`` be used?  Not when an iteration needs host work between its launches (for the H-only
+        mode on a pixel shard: the H' statistics of the ranks are combined on the host)."""
         st = self.st
         return (not (st.flags & (L.FLAG_L2 | L.FLAG_L2_H | L.FLAG_LINESEARCH)) and not self.pg_ls
-                and (self.shard is None or self.peer) and self.profile is None)
+                and (self.shard is None or (self.peer and not self.h_only)) and self.profile is None)
 
     def run_iterations(self, first, n, events=None):
         """``for it in range(first, first + n): advance(it); evaluate(it)`` issued by ONE call into the library
@@ -768,7 +821,8 @@ class FitEngine:
         iterate's buffers are intact because every kernel writes only the `next` set."""
         hp, hc, hn = self.ih
         self.ih = [hn, hp, hc]
-        self.iw = [self.iw[1], self.iw[0]]
+        if not self.h_only:                  # H-only: W / GW never rotate
+            self.iw = [self.iw[1], self.iw[0]]
         self.ihs = [self.ihs[1], self.ihs[0]]
         self.have_prev = False
         self._bind()

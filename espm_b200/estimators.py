@@ -11,15 +11,17 @@ On the device: every ``algo`` of the reference (``"log_surrogate"``, ``"l2_surro
 per phase), ``lambda_L`` with ``shape_2d`` (5-point Laplacian) or without (identity), ``fixed_H`` / ``fixed_W``,
 ``normalize``, ``linesearch``, ground-truth tracking (``true_D`` / ``true_H``), ``G`` as ``None`` / ndarray / physical
 model, ``hspy_comp``; the NNDSVD initialisation of a call without ``W`` and ``H`` runs its randomized SVD on the device
-too (``init_device.py``).  Pixel-sharded fits (one process per GPU) support every algorithm, loss and option, including
-``linesearch`` and ground-truth tracking.
+too (``init_device.py``).  With ``hspy_comp=True``, ``transform`` estimates the maps of another spectrum image with the
+fitted phases held fixed (only the H half of an iteration runs).  Pixel-sharded fits (one process per GPU) support every
+algorithm, loss and option, including ``linesearch`` and ground-truth tracking.
 """
 import sys
 import time
 
 import numpy as np
 from sklearn.base import BaseEstimator, TransformerMixin
-from sklearn.utils.validation import check_is_fitted, validate_data
+from sklearn.utils._available_if import available_if
+from sklearn.utils.validation import check_array, check_is_fitted, validate_data
 
 from . import _lib as L
 from . import config
@@ -588,6 +590,121 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
                 row += tuple(self.angles_[i]) + tuple(self.mse_[i]) + (self.true_losses_[i],)
             rows.append(row)
         return np.array(rows, dtype=dt)
+
+
+def _transform_available(est):
+    return bool(est.hspy_comp)
+
+
+def _transform(self, X, H=None, shape_2d=None):
+    """Abundance maps of a new spectrum image with the fitted phases held fixed (``hspy_comp=True`` only).
+
+    X : (p', n) array, one row per pixel (p' may differ from the fitted image), the n channels of the fitted ``G_``.
+    H : optional (k, p') initial H (internal orientation, as in ``fit_transform``).  By default
+        H0 = |lstsq(G_ W_, X)| (simplex-normalised with ``simplex_H``, clamped to ``log_shift``), computed on the device.
+    shape_2d : image shape of X for the Laplacian (``lambda_L != 0``); by default the fitted ``shape_2d`` when it
+        matches p', the identity Laplacian when the model has no ``shape_2d``.
+
+    Returns H'^T, (p', k): the H of
+    ``SmoothNMF(<same params>, G=G_, fixed_W=W_, normalize=False).fit_transform(X, W=W_, H=H)`` without its final
+    rescale.  W_ and G_ are used as fitted (a physical model is not refreshed, X is not normalised, ``fixed_H`` is
+    ignored); ``max_iter``, ``tol``, ``no_stop_criterion``, ``verbose`` and ``eval_print`` govern the loop, whose stop
+    tests and printed exits are those of the fit (with rel_W = 0).  Each iteration streams X once (the H pass).  The
+    fitted attributes are left unchanged."""
+    import copy
+    import torch
+    from .engine import FitEngine
+    from .init_device import initial_H_device
+    check_is_fitted(self, "G_")
+    for name, bad in (("algo=%r" % self.algo, self.algo in ("bmd", "projected_gradient")),
+                      ("l2=True", bool(self.l2)), ("linesearch=True", bool(self.linesearch))):
+        if bad:
+            raise NotImplementedError("SmoothNMF.transform does not support %s" % name)
+    Xv = check_array(X, dtype=[np.float64, np.float32], ensure_all_finite=False).T     # (n, p'): channels x pixels
+    n, p = Xv.shape
+    if n != self.G_.shape[0]:
+        raise ValueError("X has %d features (channels), but this SmoothNMF was fitted with %d" % (n, self.G_.shape[0]))
+    k = self.W_.shape[1]
+    if H is not None and np.shape(H) != (k, p):
+        raise ValueError("H has shape %s, expected %s" % (np.shape(H), (k, p)))
+    shape = None
+    if self.lambda_L != 0:                                   # base.py:280-291
+        from .ops import check_shape_2d
+        if shape_2d is not None:
+            shape = shape_2d
+        elif self.shape_2d is not None and int(np.prod(self.shape_2d)) == p:
+            shape = self.shape_2d
+        elif self.shape_2d is not None:
+            shape = self.shape_2d                            # check_shape_2d raises its ValueError
+        if shape is not None:
+            shape = check_shape_2d(shape, p)
+    W = self.W_
+    distributed = False
+    if config.distributed:
+        import torch.distributed as dist
+        distributed = dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1
+    shard = None
+    if distributed:
+        from .dist import make_shard
+        shard = make_shard()
+    max_iter = int(self.max_iter)
+    gamma = self.gamma if self.gamma is not None else _SIGMA_L
+    H_init = np.ones((k, p), dtype=np.result_type(W.dtype, Xv.dtype)) if H is None else np.asarray(H)
+    eng = FitEngine(Xv, None if self._identity_G else self.G_, W, H_init,
+                    shape_2d=shape, lambda_L=self.lambda_L, mu=self.mu, epsilon_reg=self.epsilon_reg,
+                    log_shift=self.log_shift, dicotomy_tol=self.dicotomy_tol, dicotomy_tol_w=_DICOTOMY_TOL,
+                    tol=self.tol, sigma=float(gamma), simplex_H=self.simplex_H, simplex_W=True,
+                    max_records=max(max_iter, 1) + 8, shard=shard, algo=self.algo, clamp_init=True, h_only=True,
+                    ingest=dict(eps=self.log_shift, normalize=None))
+    try:
+        if H is None:
+            H_init = initial_H_device(eng, self.G_, W, self.simplex_H, self.log_shift)
+            eng.set_WH(W, H_init)
+        if np.any(W < self.log_shift):
+            # the first H update uses W clamped to log_shift, every later one fixed_W itself (updates.py:75-76, 220-221)
+            eng.set_W_after_eval(W)
+            GW = W if self._identity_G else self.G_ @ W
+            if np.any(GW < self.log_shift):
+                eng.set_flag(L.FLAG_LOSS_DUAL)
+        gwf = eng.gw_flags_init()
+        if gwf & L.DEV_GW_ZERO_ROW:
+            eng.enable_clamp()
+        elif gwf & L.DEV_GW_BELOW_LS:
+            eng.set_flag(L.FLAG_LOSS_DUAL)
+        # the loop helpers record their results on the estimator they run on: give them a copy
+        run = copy.copy(self)
+        run.physics_model_ = None
+        run._track = False
+        run._engine = eng
+        run.gamma_ = gamma
+        run.const_KL_ = eng.const_KL
+        run.GWH_numel_ = n * p
+        run._init_WH = (W, H_init)
+        run.n_iter_ = 0
+        run.losses_, run.rel_, run.detailed_losses_ = [], [], []
+        algo_start = time.time()
+        batch = self.no_stop_criterion and not (self.verbose > 0 and self.eval_print > 0)
+        try:
+            if batch:
+                run._run_batch(eng, max_iter)
+            else:
+                run._run_checked(eng, max_iter, algo_start)
+        except KeyboardInterrupt:
+            pass
+        Hn = eng.get_H()
+        algo_time = time.time() - algo_start
+        print(f"Stopped after {run.n_iter_} iterations in {algo_time // 60} minutes "
+              f"and {np.round(algo_time) % 60} seconds.")
+        run._check_flags(run._final_rec)
+    finally:
+        eng.close()
+    return Hn.T
+
+
+# ``transform`` exists only with ``hspy_comp=True`` (rows of X are pixels there, as scikit-learn expects).  It is attached
+# after the class body: TransformerMixin wraps a ``transform`` defined in the class body for ``set_output``, and that
+# wrapper would make it visible on every instance.
+SmoothNMF.transform = available_if(_transform_available)(_transform)
 
 
 def register_with_espm():

@@ -212,3 +212,24 @@ def initialize_nmf_device(eng, n_components, init=None, random_state=None):
         W[W == 0] = abs(avg * rng.standard_normal(size=len(W[W == 0])) / 100)
         H[H == 0] = abs(avg * rng.standard_normal(size=len(H[H == 0])) / 100)
     return W, H
+
+
+def initial_H_device(eng, G, W, simplex_H, log_shift):
+    """The H of ``initialize_factors(X_, G, W, None, ...)`` (updates.py:207-211, 220-221) with the product against X on
+    the device: H0 = |lstsq(G W, X_)|, column-normalised when ``simplex_H``, clamped to ``log_shift``.
+
+    The pseudo-inverse of G W (k x n, the minimum-norm least-squares solution with lstsq's rank cut-off) comes from the
+    host; pinv(G W) X_ is one product with the tile-major Xt the engine holds (``_DeviceX.xt_times``, any storage type),
+    and the abs / normalise / clamp run on the k x p device result.  No host copy of X is made.  Returns a (k, p)
+    device tensor in the arithmetic type of the engine (all pixels, on every rank of a sharded engine)."""
+    X = _DeviceX(eng)
+    D = np.asarray(G, dtype=np.float64) @ np.asarray(W, dtype=np.float64)
+    pinv = np.linalg.lstsq(D, np.eye(D.shape[0]), rcond=None)[0]           # k x n, lstsq(D, .) for any right side
+    H = X.xt_times(torch.as_tensor(pinv.T.astype(_np_of(X.dtype)), device=X.device)).t().abs()   # (X_^T pinv^T)^T
+    if simplex_H:
+        H = H / H.sum(0, keepdim=True)
+    return H.clamp_min(log_shift).contiguous()
+
+
+def _np_of(dtype):
+    return np.float64 if dtype == torch.float64 else np.float32

@@ -95,6 +95,11 @@ typedef enum espm_status {
 #define ESPM_FLAG_TIMING      (1u << 22) /* diagnostics: the small kernels leave %globaltimer stamps (ns, as doubles) in
                                          * ESPM_S_T0 .. ESPM_S_T0 + 8 of the record they work on (scripts/timeline.py) */
 #define ESPM_FLAG_LINESEARCH  (1u << 18) /* smooth_nmf.py:376-386: gamma_ adapts from diff_surrogate; see sigma_dev */
+#define ESPM_FLAG_H_ONLY      (1u << 23) /* W is held fixed (fit_transform with fixed_W = W, base.py:316-324 with
+                                          * updates.py:75-76 overwriting W every iteration): espm_run_iterations only
+                                          * runs the H half of an iteration, [h_apply] -> h_stats -> h_pass -> h_finish;
+                                          * W / GW / GWc / gwstats keep the `cur` set espm_gw_prepare wrote, and the
+                                          * rel_W of every record stays 0 (SmoothNMF.transform) */
 
 /* bits of the device-side error word (espm_state.dev_flags[0]) */
 #define ESPM_DEV_NONFINITE    (1u << 0)  /* non-finite ratio sums (x/0): caller must redo with CLAMP_Y */
@@ -378,6 +383,11 @@ int espm_w_finish(const espm_state* st, void* stream);
  *       evaluate: h_pass; h_finish -> record `it` completed and stamped                   (base.py:320-324)
  * `st` is left bound to the last iterate, `lp` carries the buffer sets and the counters (in / out).  Only for fits
  * whose iteration needs nothing from the host in between (no NCCL exchange, no Gram matrices, no line search).
+ * With ESPM_FLAG_H_ONLY (W fixed) an iteration is
+ *       advance:  [h_apply]; h_stats (2 launches); rotate H / hstats only                    (base.py:316-317)
+ *       evaluate: h_pass; h_finish -> record `it` completed and stamped, rel_W left at 0
+ * i.e. 5 launches with simplex_H, 4 without, and seq_s is not advanced (there is no S exchange).  Not with
+ * ESPM_FLAG_PEER: a pixel-sharded H-only loop runs from the host, which combines the ranks' H' statistics after h_stats.
  */
 typedef struct espm_loop {
     void* H[3];              /* the three H buffers (pointers to local pixel 0) */
