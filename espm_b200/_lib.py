@@ -139,6 +139,8 @@ _EXPORTS = {
     "espm_colsum_g": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _vp]),
     "espm_h_stats": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
+    "espm_fit_stats_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.POINTER(_i64)]),
+    "espm_fit_stats": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _vp, _vp, _vp]),
     "espm_h_finish": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_apply": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),

@@ -6,6 +6,7 @@
 #include <cstdio>
 #include <cstring>
 
+#include "fitstats_decl.h"
 #include "ingest_decl.h"
 #include "small_inst.cuh"
 #include "xpass_inst.cuh"
@@ -425,6 +426,36 @@ int espm_h_pass(const espm_state* st, void* stream) {
     XPassArgs a = make_args(st, false);
     XPassLaunch l{XPASS_H, st->kp, is_safe(st) ? 1 : 0, st->h_grid, st->h_smem, h_mode(st)};
     return pick_xpass(st)(l, &a, nullptr, (cudaStream_t)stream);
+}
+
+typedef int (*fit_stats_fn)(const espm_state*, double*, double*, void*, int64_t*, cudaStream_t);
+
+static fit_stats_fn pick_fit_stats(const espm_state* st) {
+    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return fit_stats_f32f32;
+    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return fit_stats_f32f64;
+    if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) return fit_stats_f64f64;
+    if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) return fit_stats_u8f32;
+    return fit_stats_u16f32;   // check_state rejected every other pair
+}
+
+int espm_fit_stats_scratch(const espm_state* st, int64_t* bytes_out) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!bytes_out) {
+        set_error("espm_fit_stats_scratch: null output");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return pick_fit_stats(st)(st, nullptr, nullptr, nullptr, bytes_out, nullptr);
+}
+
+int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out, void* scratch, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!pixel_out || !channel_out || !scratch || !st->Xt || !st->GWc_cur || !st->H_cur) {
+        set_error("espm_fit_stats: null output, scratch or input buffer");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return pick_fit_stats(st)(st, pixel_out, channel_out, scratch, nullptr, (cudaStream_t)stream);
 }
 
 int espm_w_pass(const espm_state* st, void* stream) {

@@ -70,7 +70,8 @@ class FitEngine:
             the prologue of the reference's fit runs on the device instead of the host -- NaN / inf /
             negative checks, remove_zeros_lines (base.py:519-528), normalize (base.py:264-267) and
             const_KL_ (base.py:200-201).  Results: ``self.const_KL``, ``self.norm_factor``,
-            ``self.n_zero_rows`` / ``self.n_zero_cols``.
+            ``self.n_zero_rows`` / ``self.n_zero_cols``.  With ``check_only=True`` only the checks run: X is held as
+            given (``for_statistics``).
         h_only : W0 is held fixed and only H is iterated (``SmoothNMF.transform``, ESPM_FLAG_H_ONLY): ``advance`` runs
             [h_apply] -> h_stats and rotates the H buffers only, so an iteration streams X once (the H pass).  Only
             the multiplicative H steps (``log_surrogate`` / ``l2_surrogate``) with the KL loss.
@@ -329,6 +330,28 @@ class FitEngine:
         self.set_G(G, prepare=False)
         self._init_WH(W0, H0)
 
+    @classmethod
+    def for_statistics(cls, X, G, W, H, *, log_shift, shard=None):
+        """Engine for ``fit_statistics`` of the model (G, W, H) against X: X goes through the NaN / inf / negative checks
+        of the fit's ingest but is otherwise held as given (no remove_zeros_lines patch, no scale; uint8 / uint16 storage
+        as ``config.x_storage`` decides), and W, H are not clamped (the kernel clamps G W and H itself)."""
+        return cls(X, G, W, H, log_shift=log_shift, simplex_W=False, clamp_init=False, max_records=2, shard=shard,
+                   ingest=dict(eps=log_shift, normalize=None, check_only=True))
+
+    def fit_statistics(self):
+        """Per-pixel and per-channel sums of x, y, kl and chi2 of (W_cur, H_cur) against X (espm_fit_stats): this rank's
+        (4, p_loc) pixel block and (4, n) channel block, device float64 tensors."""
+        st, dev = self.st, self.device
+        nbytes = ctypes.c_int64(0)
+        L.check(self.lib.espm_fit_stats_scratch(ctypes.byref(st), ctypes.byref(nbytes)))
+        scratch = torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=dev)
+        pix = torch.empty(4, self.p_loc, dtype=torch.float64, device=dev)
+        chan = torch.empty(4, self.n, dtype=torch.float64, device=dev)
+        L.check(self.lib.espm_fit_stats(ctypes.byref(st), pix.data_ptr(), chan.data_ptr(), scratch.data_ptr(),
+                                        self.stream))
+        self.n_launches += 2                                 # the streaming kernel and the fold of its CTA slots
+        return pix, chan
+
     # ------------------------------------------------------------------ helpers
     @property
     def stream(self):
@@ -465,7 +488,8 @@ class FitEngine:
                               col_nz.sum().reshape(1).to(torch.int32)]).cpu().numpy()
             flags = int(info[0]) & 0xffffffff
             vmax = float(np.array([info[1]], dtype=np.int32).view(np.float32)[0])
-            patched = ingest is not None and (int(info[2]) < self.n or int(info[3]) < self.p_loc)
+            patched = (ingest is not None and not ingest.get("check_only")
+                       and (int(info[2]) < self.n or int(info[3]) < self.p_loc))
             if flags & (L.X_NAN | L.X_INF | L.X_NEGATIVE | L.X_FRACTION) or patched:
                 want = 2                                   # (errors are raised by the ingest pass, with its messages)
                 self.x_storage_reason = "non-integer / negative entries or all-zero lines"
@@ -496,10 +520,11 @@ class FitEngine:
                                            self.stream))
             torch.cuda.current_stream(self.device).synchronize()
         else:
-            self._ingest(src, sc, sp, float(ingest.get("eps", st.log_shift)), ingest.get("normalize"))
+            self._ingest(src, sc, sp, float(ingest.get("eps", st.log_shift)), ingest.get("normalize"),
+                         bool(ingest.get("check_only")))
         self._xraw = None
 
-    def _ingest(self, src, sc, sp, eps, normalize_nc):
+    def _ingest(self, src, sc, sp, eps, normalize_nc, ingest_only_checks=False):
         """Device-side prologue of the fit (see ``ingest`` in __init__)."""
         st, dev = self.st, self.device
         i32 = torch.int32
@@ -526,6 +551,8 @@ class FitEngine:
                              % np.dtype(_np_dtype(self.src_code)).name)
         if flags & L.X_NEGATIVE:
             raise ValueError("Negative values in data")            # base.py:528
+        if ingest_only_checks:
+            return
         total = float(info[1])
         zc = int(round(info[2]))
         zr = int(n - int(row_nz[:n].sum().item()))

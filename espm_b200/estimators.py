@@ -12,11 +12,13 @@ per phase), ``lambda_L`` with ``shape_2d`` (5-point Laplacian) or without (ident
 ``normalize``, ``linesearch``, ground-truth tracking (``true_D`` / ``true_H``), ``G`` as ``None`` / ndarray / physical
 model, ``hspy_comp``; the NNDSVD initialisation of a call without ``W`` and ``H`` runs its randomized SVD on the device
 too (``init_device.py``).  With ``hspy_comp=True``, ``transform`` estimates the maps of another spectrum image with the
-fitted phases held fixed (only the H half of an iteration runs).  Pixel-sharded fits (one process per GPU) support every
+fitted phases held fixed (only the H half of an iteration runs).  ``goodness_of_fit`` maps where a fitted model
+explains the data and where it does not (per-pixel and per-channel KL and chi-square sums, one pass over X).  Pixel-sharded fits (one process per GPU) support every
 algorithm, loss and option, including ``linesearch`` and ground-truth tracking.
 """
 import sys
 import time
+from collections import namedtuple
 
 import numpy as np
 from sklearn.base import BaseEstimator, TransformerMixin
@@ -30,6 +32,16 @@ from .conf import log_shift as _LOG_SHIFT
 from .conf import sigmaL as _SIGMA_L
 from .host import (find_min_angle, find_min_MSE, initialize_factors, is_physical_model, normalization_factor,
                    remove_zeros_lines, rescaled_DH)
+
+
+FitStatistics = namedtuple("FitStatistics", ["pixel_counts", "pixel_model", "pixel_kl", "pixel_chi2",
+                                             "channel_counts", "channel_model", "channel_kl", "channel_chi2"])
+FitStatistics.__doc__ = """Goodness of fit of a SmoothNMF model (``SmoothNMF.goodness_of_fit``), float64 arrays.
+
+With x the data, y = sum_k max(GW, log_shift) max(H, log_shift) the model (the Y of the KL loss),
+kl = y - x + x ln(x / y) (0 ln 0 := 0) and chi2 = (x - y)^2 / y:
+``pixel_*`` (p,) are the sums over channels of x, y, kl, chi2 for every pixel (pixel order of the X passed in),
+``channel_*`` (n,) the sums over pixels for every channel."""
 
 
 class SmoothNMF(TransformerMixin, BaseEstimator):
@@ -568,6 +580,63 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         """Learn the model (base.py:422-441)."""
         self.fit_transform(X, **params)
         return self
+
+    def goodness_of_fit(self, X, H=None):
+        """Where the fitted model explains X and where it does not: per-pixel and per-channel sums of the counts, the
+        model, the KL divergence and Pearson's chi-square, computed on the device in one pass over X.
+
+        X : the data, laid out as for ``fit_transform`` ((n, p), or (p, n) with ``hspy_comp=True``), with the n channels
+            of the fitted ``G_``.  Used as given: zero lines are not patched and nothing is normalised; NaN, inf and
+            negative entries raise the errors of ``fit``.
+        H : (k, p) maps in the internal orientation, e.g. ``est.transform(X_b).T`` for a new image; by default the
+            fitted ``H_`` (X must then have the fitted pixel count).
+
+        The model is ``G_ W_ H`` with the fitted ``W_`` (already on the scale of the raw data when ``normalize=True``) and
+        ``G_`` as fitted.  ``algo``, ``l2`` and the regularisers play no part.  Returns a ``FitStatistics``; the residual
+        sum spectrum is ``channel_counts - channel_model``.  Leaves every fitted attribute unchanged.  In a pixel-sharded
+        run every rank passes the whole X and gets the whole, identical, result."""
+        import torch
+        from .engine import FitEngine
+        check_is_fitted(self, "G_")
+        Xa = check_array(X, dtype=[np.float64, np.float32], ensure_all_finite=False)
+        Xv = Xa.T if self.hspy_comp else Xa                       # (n, p): channels x pixels
+        n, p = Xv.shape
+        if n != self.G_.shape[0]:
+            raise ValueError("X has %d channels, but this SmoothNMF was fitted with %d" % (n, self.G_.shape[0]))
+        k = self.W_.shape[1]
+        if H is None:
+            if p != self.H_.shape[1]:
+                raise ValueError("X has %d pixels but the fitted H_ has %d: pass the maps of this image as H"
+                                 % (p, self.H_.shape[1]))
+            H = self.H_
+        elif np.shape(H) != (k, p):
+            raise ValueError("H has shape %s, expected %s" % (np.shape(H), (k, p)))
+        shard = None
+        if config.distributed:
+            import torch.distributed as dist
+            if dist.is_available() and dist.is_initialized() and dist.get_world_size() > 1:
+                from .dist import make_shard
+                shard = make_shard()
+        eng = FitEngine.for_statistics(Xv, None if self._identity_G else self.G_, self.W_, np.asarray(H),
+                                       log_shift=self.log_shift, shard=shard)
+        try:
+            pix, chan = eng.fit_statistics()
+            if shard is None:
+                pix, chan = pix.cpu().numpy(), chan.cpu().numpy()
+            else:
+                import torch.distributed as dist
+                from .dist import shard_bounds
+                parts = [torch.empty_like(chan) for _ in range(shard.world)]
+                dist.all_gather(parts, chan, group=shard.group)
+                for r in range(1, shard.world):               # rank order: the same bits on every rank
+                    parts[0] += parts[r]
+                chan = parts[0].cpu().numpy()
+                sizes = [b - a for a, b, _ in (shard_bounds(p, eng.nx, eng.ny, r, shard.world)
+                                              for r in range(shard.world))]
+                pix = shard.gather_H_device(pix, sizes)
+        finally:
+            eng.close()
+        return FitStatistics(*pix, *chan)
 
     def inverse_transform(self, W):
         """G W H (base.py:461-477)."""

@@ -188,7 +188,8 @@ typedef struct espm_state {
     const void* W_cur;      /* m x k row-major */
     void* W_next;
     const void* GW_cur;     /* n_pad x kp */
-    const void* GWc_cur;    /* max(GW, ls), n_pad x kp (only read when ESPM_FLAG_LOSS_DUAL) */
+    const void* GWc_cur;    /* max(GW, ls), n_pad x kp (written by every espm_gw_prepare; read by the X passes only with
+                             * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats) */
     void* GW_next;
     void* GWc_next;
     void* gwstats_cur;      /* 2*kp (c dtype): colsum(GW), colsum(max(GW,ls)) over the n real rows */
@@ -352,6 +353,17 @@ int espm_h_stats(const espm_state* st, void* stream);
  *   xlogy_part[cta] = partial of sum max(X,ls)*log(Y) for (GW_cur, H_cur)
  */
 int espm_h_pass(const espm_state* st, void* stream);
+/*
+ * Goodness of fit of (GW_cur, H_cur) against Xt over this rank's pixels (SmoothNMF.goodness_of_fit), one pass over Xt:
+ *   y = sum_k max(GW, ls) max(H, ls),  kl = y - x + x ln(x / y) (x ln x := 0 at x == 0),  chi2 = (x - y)^2 / y
+ *   pixel_out   [4][p_loc] doubles: per pixel sum over the n channels of x, y, kl, chi2
+ *   channel_out [4][n]     doubles: per channel sum over this rank's pixels, folded in a fixed order
+ *   scratch: espm_fit_stats_scratch() bytes of device memory owned by the caller.
+ * Reads Xt, GWc_cur (= max(GW_cur, ls), written with GW_cur by espm_gw_prepare), H_cur (k x ldh) and log_shift; writes
+ * no record and no device flag.  Deterministic: two calls give identical bits.
+ */
+int espm_fit_stats_scratch(const espm_state* st, int64_t* bytes_out);
+int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out, void* scratch, void* stream);
 /*
  * Per-pixel assembly (updates.py:132-142): num, den with the log and Laplacian surrogates, the loss
  * regularisers of the CURRENT iterate (measures.py:548,577), rel_H (base.py:324), and either
