@@ -7,6 +7,7 @@
 #include <cstring>
 
 #include "fitstats_decl.h"
+#include "hinfo_decl.h"
 #include "ingest_decl.h"
 #include "small_inst.cuh"
 #include "xpass_inst.cuh"
@@ -456,6 +457,23 @@ int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out,
         return ESPM_ERR_BAD_ARG;
     }
     return pick_fit_stats(st)(st, pixel_out, channel_out, scratch, nullptr, (cudaStream_t)stream);
+}
+
+typedef int (*h_info_fn)(const espm_state*, int, double*, cudaStream_t);
+
+int espm_abundance_info(const espm_state* st, int simplex, double* out, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!out || !st->Xt || !st->GWc_cur || !st->H_cur) {
+        set_error("espm_abundance_info: null output or input buffer");
+        return ESPM_ERR_BAD_ARG;
+    }
+    h_info_fn fn = h_info_u16f32;   // check_state rejected every other pair
+    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) fn = h_info_f32f32;
+    else if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) fn = h_info_f32f64;
+    else if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) fn = h_info_f64f64;
+    else if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) fn = h_info_u8f32;
+    return fn(st, simplex ? 1 : 0, out, (cudaStream_t)stream);
 }
 
 int espm_w_pass(const espm_state* st, void* stream) {

@@ -352,6 +352,16 @@ class FitEngine:
         self.n_launches += 2                                 # the streaming kernel and the fold of its CTA slots
         return pix, chan
 
+    def abundance_information(self, simplex):
+        """Poisson information F_j and covariance C_j of H_cur's columns given W_cur (espm_abundance_info): this rank's
+        (k + k(k+1), p_loc) device float64 tensor of the k std rows, then C and F as packed upper triangles, row by row.
+        ``simplex`` projects C onto sum_a h_aj = 1."""
+        k = self.k
+        out = torch.empty(k + k * (k + 1), self.p_loc, dtype=torch.float64, device=self.device)
+        L.check(self.lib.espm_abundance_info(ctypes.byref(self.st), 1 if simplex else 0, out.data_ptr(), self.stream))
+        self.n_launches += 2                                 # the streaming kernel and the per-pixel inversion
+        return out
+
     # ------------------------------------------------------------------ helpers
     @property
     def stream(self):

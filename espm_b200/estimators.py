@@ -13,7 +13,9 @@ per phase), ``lambda_L`` with ``shape_2d`` (5-point Laplacian) or without (ident
 model, ``hspy_comp``; the NNDSVD initialisation of a call without ``W`` and ``H`` runs its randomized SVD on the device
 too (``init_device.py``).  With ``hspy_comp=True``, ``transform`` estimates the maps of another spectrum image with the
 fitted phases held fixed (only the H half of an iteration runs).  ``goodness_of_fit`` maps where a fitted model
-explains the data and where it does not (per-pixel and per-channel KL and chi-square sums, one pass over X).  Pixel-sharded fits (one process per GPU) support every
+explains the data and where it does not (per-pixel and per-channel KL and chi-square sums, one pass over X), and
+``abundance_uncertainty`` how precise the maps are (per-pixel standard errors and covariances from the Poisson
+information, one pass over X).  Pixel-sharded fits (one process per GPU) support every
 algorithm, loss and option, including ``linesearch`` and ground-truth tracking.
 """
 import sys
@@ -42,6 +44,12 @@ With x the data, y = sum_k max(GW, log_shift) max(H, log_shift) the model (the Y
 kl = y - x + x ln(x / y) (0 ln 0 := 0) and chi2 = (x - y)^2 / y:
 ``pixel_*`` (p,) are the sums over channels of x, y, kl, chi2 for every pixel (pixel order of the X passed in),
 ``channel_*`` (n,) the sums over pixels for every channel."""
+
+AbundanceUncertainty = namedtuple("AbundanceUncertainty", ["std", "covariance", "information"])
+AbundanceUncertainty.__doc__ = """Precision of the abundance maps of a SmoothNMF model (``SmoothNMF.abundance_uncertainty``), float64
+arrays: ``std`` (k, p) the standard error of every entry of H, ``covariance`` (p, k, k) the covariance of every pixel's
+column of H and ``information`` (p, k, k) its Poisson information matrix (both symmetric).  NaN ``std`` and
+``covariance`` mark a pixel whose information is singular."""
 
 
 class SmoothNMF(TransformerMixin, BaseEstimator):
@@ -596,6 +604,66 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         sum spectrum is ``channel_counts - channel_model``.  Leaves every fitted attribute unchanged.  In a pixel-sharded
         run every rank passes the whole X and gets the whole, identical, result."""
         import torch
+        eng, shard, p = self._statistics_engine(X, H)
+        try:
+            pix, chan = eng.fit_statistics()
+            if shard is None:
+                pix, chan = pix.cpu().numpy(), chan.cpu().numpy()
+            else:
+                import torch.distributed as dist
+                parts = [torch.empty_like(chan) for _ in range(shard.world)]
+                dist.all_gather(parts, chan, group=shard.group)
+                for r in range(1, shard.world):               # rank order: the same bits on every rank
+                    parts[0] += parts[r]
+                chan = parts[0].cpu().numpy()
+                pix = self._gather_pixels(eng, shard, p, pix)
+        finally:
+            eng.close()
+        return FitStatistics(*pix, *chan)
+
+    def abundance_uncertainty(self, X, H=None):
+        """Standard errors and covariances of the abundance maps, per pixel, from the Poisson information of X given the
+        fitted phases, computed on the device in one pass over X.
+
+        With g = max(G_ W_, log_shift), h = max(H, log_shift) and y = g h (the clamped model of the KL loss), pixel j's
+        information is F_j[a, b] = sum_c x_cj g_ca g_cb / y_cj^2, the Hessian of the KL loss in the column H[:, j].  Its
+        covariance is C_j = F_j^-1, and with ``simplex_H=True`` the covariance under sum_a h_aj = 1,
+        C_j = F_j^-1 - (F_j^-1 1)(F_j^-1 1)^T / (1^T F_j^-1 1) (so C_j 1 = 0); ``std`` is sqrt(diag C_j).
+
+        This is the Poisson (likelihood, Cramer-Rao) bound given the fitted phases G_ W_, which are treated as exact.  It is
+        not a posterior of the regularised objective: ``lambda_L``, ``mu`` and ``epsilon_reg`` play no part, nor do
+        ``algo`` and ``l2``.  Where a phase sits on the ``log_shift`` bound the bound treats that phase as free.
+
+        X : the data, laid out as for ``fit_transform`` ((n, p), or (p, n) with ``hspy_comp=True``), with the n channels
+            of the fitted ``G_``.  Used as given: zero lines are not patched and nothing is normalised; NaN, inf and
+            negative entries raise the errors of ``fit``.
+        H : (k, p) maps in the internal orientation, e.g. ``est.transform(X_b).T`` for a new image; by default the
+            fitted ``H_`` (X must then have the fitted pixel count).
+
+        Returns an ``AbundanceUncertainty`` of float64 arrays: ``std`` (k, p), ``covariance`` and ``information``
+        (p, k, k).  A pixel whose F_j is singular (a Cholesky pivot <= 1e-12 max_a F_j[a, a], e.g. a pixel without
+        counts) gets NaN ``std`` and ``covariance``; its ``information`` is returned all the same.  Nothing is printed and
+        no fitted attribute changes.  In a pixel-sharded run every rank passes the whole X and gets the whole, identical,
+        result."""
+        eng, shard, p = self._statistics_engine(X, H)
+        try:
+            out = eng.abundance_information(bool(self.simplex_H))
+            out = out.cpu().numpy() if shard is None else self._gather_pixels(eng, shard, p, out)
+        finally:
+            eng.close()
+        k = eng.k
+        iu = np.triu_indices(k)
+        cov = np.empty((p, k, k))
+        info = np.empty((p, k, k))
+        nt = iu[0].size
+        for full, rows in ((cov, out[k:k + nt]), (info, out[k + nt:])):
+            full[:, iu[0], iu[1]] = rows.T
+            full[:, iu[1], iu[0]] = rows.T
+        return AbundanceUncertainty(np.ascontiguousarray(out[:k]), cov, info)
+
+    def _statistics_engine(self, X, H):
+        """Checks the arguments of goodness_of_fit / abundance_uncertainty (before any device work) and builds the
+        FitEngine of the fitted model against X: (engine, shard or None, pixel count)."""
         from .engine import FitEngine
         check_is_fitted(self, "G_")
         Xa = check_array(X, dtype=[np.float64, np.float32], ensure_all_finite=False)
@@ -619,24 +687,14 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
                 shard = make_shard()
         eng = FitEngine.for_statistics(Xv, None if self._identity_G else self.G_, self.W_, np.asarray(H),
                                        log_shift=self.log_shift, shard=shard)
-        try:
-            pix, chan = eng.fit_statistics()
-            if shard is None:
-                pix, chan = pix.cpu().numpy(), chan.cpu().numpy()
-            else:
-                import torch.distributed as dist
-                from .dist import shard_bounds
-                parts = [torch.empty_like(chan) for _ in range(shard.world)]
-                dist.all_gather(parts, chan, group=shard.group)
-                for r in range(1, shard.world):               # rank order: the same bits on every rank
-                    parts[0] += parts[r]
-                chan = parts[0].cpu().numpy()
-                sizes = [b - a for a, b, _ in (shard_bounds(p, eng.nx, eng.ny, r, shard.world)
-                                              for r in range(shard.world))]
-                pix = shard.gather_H_device(pix, sizes)
-        finally:
-            eng.close()
-        return FitStatistics(*pix, *chan)
+        return eng, shard, p
+
+    @staticmethod
+    def _gather_pixels(eng, shard, p, block):
+        """The (rows, p) host array of every rank's (rows, p_loc) device block, in rank order, identical on all ranks."""
+        from .dist import shard_bounds
+        sizes = [b - a for a, b, _ in (shard_bounds(p, eng.nx, eng.ny, r, shard.world) for r in range(shard.world))]
+        return shard.gather_H_device(block, sizes)
 
     def inverse_transform(self, W):
         """G W H (base.py:461-477)."""

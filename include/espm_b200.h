@@ -189,7 +189,8 @@ typedef struct espm_state {
     void* W_next;
     const void* GW_cur;     /* n_pad x kp */
     const void* GWc_cur;    /* max(GW, ls), n_pad x kp (written by every espm_gw_prepare; read by the X passes only with
-                             * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats) */
+                             * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats and
+                             * espm_abundance_info) */
     void* GW_next;
     void* GWc_next;
     void* gwstats_cur;      /* 2*kp (c dtype): colsum(GW), colsum(max(GW,ls)) over the n real rows */
@@ -364,6 +365,21 @@ int espm_h_pass(const espm_state* st, void* stream);
  */
 int espm_fit_stats_scratch(const espm_state* st, int64_t* bytes_out);
 int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out, void* scratch, void* stream);
+/*
+ * Poisson information and covariance of the abundance maps H_cur given (GW_cur) over this rank's pixels
+ * (SmoothNMF.abundance_uncertainty), one pass over Xt:
+ *   y_cj     = sum_a g_ca h_aj,   g = max(GW, ls), h = max(H, ls)            (the clamped Y of the KL loss)
+ *   F_j[a,b] = sum_c x_cj g_ca g_cb / y_cj^2                                  (Hessian of the KL loss in H[:, j])
+ *   C_j      = F_j^-1                                                         simplex == 0
+ *   C_j      = F_j^-1 - (F_j^-1 1)(F_j^-1 1)^T / (1^T F_j^-1 1)              simplex != 0 (sum_a h_aj = 1; C_j 1 = 0)
+ *   std_aj   = sqrt(C_j[a,a])
+ * out: [k + 2 k (k + 1) / 2][p_loc] doubles: the k std rows, then C, then F, each symmetric matrix as its packed upper
+ * triangle row by row ((0,0), (0,1), ..., (0,k-1), (1,1), ...).  A pixel whose F_j meets a Cholesky pivot
+ * <= 1e-12 max_a F_j[a,a] (or is zero: no counts) gets NaN std and C; its F is written all the same.
+ * Reads Xt, GWc_cur, H_cur (k x ldh) and log_shift; writes no record and no device flag.  No atomics, fixed summation
+ * order: two calls give identical bits, and a pixel shard gives the bits of the whole image.  Two launches.
+ */
+int espm_abundance_info(const espm_state* st, int simplex, double* out, void* stream);
 /*
  * Per-pixel assembly (updates.py:132-142): num, den with the log and Laplacian surrogates, the loss
  * regularisers of the CURRENT iterate (measures.py:548,577), rel_H (base.py:324), and either
