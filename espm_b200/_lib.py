@@ -142,6 +142,8 @@ _EXPORTS = {
     "espm_fit_stats_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.POINTER(_i64)]),
     "espm_fit_stats": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _vp, _vp, _vp]),
     "espm_abundance_info": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.c_int, _vp, _vp]),
+    "espm_phase_info_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.POINTER(_i64)]),
+    "espm_phase_info": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _vp, _vp]),
     "espm_h_finish": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_apply": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),

@@ -10,6 +10,7 @@
 #include "hinfo_decl.h"
 #include "ingest_decl.h"
 #include "small_inst.cuh"
+#include "winfo_decl.h"
 #include "xpass_inst.cuh"
 
 namespace espm {
@@ -474,6 +475,36 @@ int espm_abundance_info(const espm_state* st, int simplex, double* out, void* st
     else if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) fn = h_info_f64f64;
     else if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) fn = h_info_u8f32;
     return fn(st, simplex ? 1 : 0, out, (cudaStream_t)stream);
+}
+
+typedef int (*w_info_fn)(const espm_state*, double*, void*, int64_t*, cudaStream_t);
+
+static w_info_fn pick_w_info(const espm_state* st) {
+    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return w_info_f32f32;
+    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return w_info_f32f64;
+    if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) return w_info_f64f64;
+    if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) return w_info_u8f32;
+    return w_info_u16f32;   // check_state rejected every other pair
+}
+
+int espm_phase_info_scratch(const espm_state* st, int64_t* bytes_out) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!bytes_out) {
+        set_error("espm_phase_info_scratch: null output");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return pick_w_info(st)(st, nullptr, nullptr, bytes_out, nullptr);
+}
+
+int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stream) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (!out || !scratch || !st->Xt || !st->GWc_cur || !st->H_cur) {
+        set_error("espm_phase_info: null output, scratch or input buffer");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return pick_w_info(st)(st, out, scratch, nullptr, (cudaStream_t)stream);
 }
 
 int espm_w_pass(const espm_state* st, void* stream) {

@@ -362,6 +362,18 @@ class FitEngine:
         self.n_launches += 2                                 # the streaming kernel and the per-pixel inversion
         return out
 
+    def phase_information(self):
+        """Poisson information of the phases per channel given H_cur (espm_phase_info): this rank's (k(k+1)/2, n) device
+        float64 tensor of A_c[a, b] = sum_j x_cj h_aj h_bj / y_cj^2 as packed upper triangles, row by row."""
+        st, dev = self.st, self.device
+        nbytes = ctypes.c_int64(0)
+        L.check(self.lib.espm_phase_info_scratch(ctypes.byref(st), ctypes.byref(nbytes)))
+        scratch = torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=dev)
+        out = torch.empty(self.k * (self.k + 1) // 2, self.n, dtype=torch.float64, device=dev)
+        L.check(self.lib.espm_phase_info(ctypes.byref(st), out.data_ptr(), scratch.data_ptr(), self.stream))
+        self.n_launches += 3                                 # the H tiles, the streaming kernel and the fold of its slots
+        return out
+
     # ------------------------------------------------------------------ helpers
     @property
     def stream(self):

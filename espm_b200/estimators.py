@@ -15,7 +15,8 @@ too (``init_device.py``).  With ``hspy_comp=True``, ``transform`` estimates the 
 fitted phases held fixed (only the H half of an iteration runs).  ``goodness_of_fit`` maps where a fitted model
 explains the data and where it does not (per-pixel and per-channel KL and chi-square sums, one pass over X), and
 ``abundance_uncertainty`` how precise the maps are (per-pixel standard errors and covariances from the Poisson
-information, one pass over X).  Pixel-sharded fits (one process per GPU) support every
+information, one pass over X), and ``phase_uncertainty`` how precise the phases are (standard errors and covariances of
+``W_`` and error bands of the phase spectra, from the per-channel Poisson information, one pass over X).  Pixel-sharded fits (one process per GPU) support every
 algorithm, loss and option, including ``linesearch`` and ground-truth tracking.
 """
 import sys
@@ -50,6 +51,14 @@ AbundanceUncertainty.__doc__ = """Precision of the abundance maps of a SmoothNMF
 arrays: ``std`` (k, p) the standard error of every entry of H, ``covariance`` (p, k, k) the covariance of every pixel's
 column of H and ``information`` (p, k, k) its Poisson information matrix (both symmetric).  NaN ``std`` and
 ``covariance`` mark a pixel whose information is singular."""
+
+PhaseUncertainty = namedtuple("PhaseUncertainty", ["std", "covariance", "information", "spectrum_std"])
+PhaseUncertainty.__doc__ = """Precision of the phases of a SmoothNMF model (``SmoothNMF.phase_uncertainty``), float64 arrays.
+With a real G (n x m): ``std`` (m, k) the standard error of every entry of W, ``covariance`` and ``information`` (m, k,
+m, k) the covariance and Poisson information of vec(W).  With G = None (m = n): ``std`` (n, k) and the diagonal blocks
+only, ``covariance`` and ``information`` (n, k, k), one per channel.  ``spectrum_std`` (n, k) is the standard error of
+the phase spectra G W (``components_``).  NaN marks singular information: all of std, covariance and spectrum_std with a
+real G, the channel's entries with G = None."""
 
 
 class SmoothNMF(TransformerMixin, BaseEstimator):
@@ -661,9 +670,63 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
             full[:, iu[1], iu[0]] = rows.T
         return AbundanceUncertainty(np.ascontiguousarray(out[:k]), cov, info)
 
+    def phase_uncertainty(self, X, H=None):
+        """Standard errors and covariances of the phases W_ from the Poisson information of X given the maps, with the
+        per-channel sums computed on the device in one pass over X and the small algebra on the host in fp64.
+
+        With g = max(G_ W_, log_shift), h = max(H, log_shift) and y = g h (the clamped model of the KL loss), channel c
+        contributes A_c[a, b] = sum_j x_cj h_aj h_bj / y_cj^2, and the information of vec(W), index (e, a), is
+        F[(e,a),(f,b)] = sum_c G_ce G_cf A_c[a, b] (with G = None, G is the identity and F is block diagonal with blocks
+        A_c).  The covariance is the constrained Cramer-Rao bound on the free entries phi = {(e, a): fixed_W is None or
+        fixed_W[e, a] < 0}: with ``simplex_W`` one constraint sum_{e in S} W_ea = const per column a over its free
+        entries, S = ``physics_model_.NMF_simplex()`` for a physical model and every row otherwise, and with constraint
+        matrix A, C = F^-1 - F^-1 A^T (A F^-1 A^T)^-1 A F^-1.  ``std`` is sqrt(diag C) and ``spectrum_std[c, a]`` =
+        sqrt(sum_{e,f} G_ce G_cf C[(e,a),(f,a)]), the error band of the phase spectra G W (``components_``).  Fixed
+        entries have std 0 and zero covariance.
+
+        This is the Poisson (likelihood) bound with the maps H held fixed and treated as exact.  It is not a posterior of
+        the regularised objective: ``lambda_L``, ``mu``, ``epsilon_reg``, ``algo`` and ``l2`` play no part.
+
+        X : the data, laid out as for ``fit_transform``, with the n channels of the fitted ``G_``.  Used as given; NaN,
+            inf and negative entries raise the errors of ``fit``.
+        H : (k, p) maps in the internal orientation, e.g. ``est.transform(X_b).T`` for a new image; by default the
+            fitted ``H_``.
+
+        Returns a ``PhaseUncertainty``.  With a real G, ``std`` is (m, k) and ``covariance`` and ``information`` the full
+        (m, k, m, k) matrices; with G = None, ``std`` is (n, k) and ``covariance`` and ``information`` are the (n, k, k)
+        diagonal blocks (the full nk x nk matrix would take gigabytes); with ``simplex_W`` a block is B_c - B_c M^-1 B_c,
+        B_c = A_c^-1 on the free phases and M = sum_c B_c.  ``spectrum_std`` is (n, k).  Singular information (a
+        Cholesky pivot <= 1e-12 of the largest diagonal entry) is NaN: with a real G all of std, covariance and
+        spectrum_std; with G = None only that channel (e.g. one without counts), which is then left out of M, as a fixed
+        entry is.  ``information`` is always returned.  Nothing is printed and no fitted attribute changes.  In a
+        pixel-sharded run every rank passes the whole X and gets the whole, identical, result."""
+        import torch
+        from .host import phase_covariance
+        eng, shard, _ = self._statistics_engine(X, H)
+        try:
+            A = eng.phase_information()
+            if shard is not None:
+                import torch.distributed as dist
+                parts = [torch.empty_like(A) for _ in range(shard.world)]
+                dist.all_gather(parts, A, group=shard.group)
+                for r in range(1, shard.world):               # rank order: the same bits on every rank
+                    parts[0] += parts[r]
+                A = parts[0]
+            A = A.cpu().numpy()
+        finally:
+            eng.close()
+        m, k = self.W_.shape
+        # the projected gradient fit passes no fixed_W to its updates (smooth_nmf.py:430-437)
+        fixed = None if self.algo == "projected_gradient" else self.fixed_W
+        free = np.ones((m, k), dtype=bool) if fixed is None else np.asarray(fixed) < 0
+        rows = None
+        if self.simplex_W:
+            rows = np.arange(m) if self.physics_model_ is None else np.asarray(self.physics_model_.NMF_simplex())
+        return PhaseUncertainty(*phase_covariance(A, None if self._identity_G else self.G_, free, rows))
+
     def _statistics_engine(self, X, H):
-        """Checks the arguments of goodness_of_fit / abundance_uncertainty (before any device work) and builds the
-        FitEngine of the fitted model against X: (engine, shard or None, pixel count)."""
+        """Checks the arguments of goodness_of_fit / abundance_uncertainty / phase_uncertainty (before any device work)
+        and builds the FitEngine of the fitted model against X: (engine, shard or None, pixel count)."""
         from .engine import FitEngine
         check_is_fitted(self, "G_")
         Xa = check_array(X, dtype=[np.float64, np.float32], ensure_all_finite=False)

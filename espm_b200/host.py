@@ -124,3 +124,116 @@ def find_min_MSE(true_maps, algo_maps):
     xy = np.dot(true_maps, algo_maps.T)
     d = abs(np.kron(np.ones((algo_maps.shape[0], 1)), xx).T + np.kron(np.ones((true_maps.shape[0], 1)), yy) - 2 * xy)
     return _unique_min(d / true_maps.shape[1])[0]
+
+
+# ---- SmoothNMF.phase_uncertainty: covariance of W from the per-channel information the device computes ------------
+PIVOT_REL = 1e-12      # a Cholesky pivot <= PIVOT_REL max diag marks the information singular (as hinfo.cuh)
+
+
+def _cholesky(F):
+    """Lower Cholesky factor of F, or None when F is singular: an all-zero diagonal, a failed factorisation or a pivot
+    L_ii^2 <= PIVOT_REL max_i F_ii."""
+    dmax = float(np.max(np.diag(F))) if F.size else 0.0
+    if not dmax > 0.0:
+        return None
+    try:
+        L = np.linalg.cholesky(F)
+    except np.linalg.LinAlgError:
+        return None
+    return L if np.min(np.diag(L)) ** 2 > PIVOT_REL * dmax else None
+
+
+def _inverse(F):
+    from scipy.linalg import cho_solve
+    L = _cholesky(F)
+    return None if L is None else cho_solve((L, True), np.eye(F.shape[0]))
+
+
+def unpack_triangles(packed, k):
+    """(k(k+1)/2, n) packed upper triangles, row by row -> (n, k, k) symmetric matrices."""
+    iu = np.triu_indices(k)
+    out = np.empty((packed.shape[1], k, k))
+    out[:, iu[0], iu[1]] = packed.T
+    out[:, iu[1], iu[0]] = packed.T
+    return out
+
+
+def phase_covariance(A_packed, G, free, simplex_rows):
+    """Constrained Cramer-Rao bound of the phases W (m x k) from the per-channel information of the device.
+
+    A_packed : (k(k+1)/2, n) A_c[a, b] = sum_j x_cj h_aj h_bj / y_cj^2, packed upper triangles row by row.
+    G : (n, m) or None for the identity (m = n).
+    free : (m, k) bool, the entries of W the fit updates.
+    simplex_rows : None, or the rows S of W whose column sums the fit holds: one constraint sum_{e in S} W_ea = const per
+        column a over its free entries (dropped when it has none).
+
+    The information of vec(W), index (e, a), is F[(e,a),(f,b)] = sum_c G_ce G_cf A_c[a, b]; on the free entries
+    C = F^-1 - F^-1 A^T (A F^-1 A^T)^-1 A F^-1 for the constraint matrix A.  Returns (std, covariance, information,
+    spectrum_std), float64:
+      real G: std (m, k), covariance and information (m, k, m, k), spectrum_std (n, k) with
+              spectrum_std[c, a]^2 = sum_{e,f} G_ce G_cf C[(e,a),(f,a)]; a singular F makes std, covariance and
+              spectrum_std all NaN;
+      G None: F is block diagonal (blocks A_c), and only the blocks are returned: std (n, k), covariance and information
+              (n, k, k), spectrum_std = std.  With B_c = A_c^-1 on the free phases of channel c and M = sum_{c in S} B_c,
+              the block of C is B_c - B_c M^-1 B_c (no dense nk x nk matrix is formed).  A channel with singular A_c is
+              NaN and is left out of M, as a fixed entry is.
+    Fixed entries have std 0 and zero covariance rows."""
+    nt, n = A_packed.shape
+    k = int(round((np.sqrt(8 * nt + 1) - 1) / 2))
+    A = unpack_triangles(np.asarray(A_packed, dtype=np.float64), k)
+    free = np.asarray(free, dtype=bool)
+    if G is None:
+        return _block_covariance(A, free, simplex_rows)
+    G = np.asarray(G, dtype=np.float64)
+    m = G.shape[1]
+    GG = (G[:, :, None] * G[:, None, :]).reshape(n, m * m)
+    F = (GG.T @ A.reshape(n, k * k)).reshape(m, m, k, k).transpose(0, 2, 1, 3).reshape(m * k, m * k)
+    phi = np.flatnonzero(free.reshape(-1))
+    C = np.zeros((m * k, m * k))
+    if phi.size:
+        Fi = _inverse(F[np.ix_(phi, phi)])
+        if Fi is None:
+            nan = np.full((m, k), np.nan)
+            return nan, np.full((m, k, m, k), np.nan), F.reshape(m, k, m, k), np.full((n, k), np.nan)
+        if simplex_rows is not None:
+            in_S = np.zeros(m, dtype=bool)
+            in_S[np.asarray(simplex_rows, dtype=np.int64)] = True
+            rows = [(in_S[:, None] & free & (np.arange(k) == a)[None, :]).reshape(-1)[phi] for a in range(k)]
+            Acon = np.array([r for r in rows if r.any()], dtype=np.float64).reshape(-1, phi.size)
+            if Acon.shape[0]:
+                B = Fi @ Acon.T
+                Fi = Fi - B @ np.linalg.solve(Acon @ B, B.T)
+        C[np.ix_(phi, phi)] = 0.5 * (Fi + Fi.T)
+    C = C.reshape(m, k, m, k)
+    std = np.sqrt(np.maximum(np.einsum("eaea->ea", C), 0.0))
+    spec = np.stack([((G @ C[:, a, :, a]) * G).sum(1) for a in range(k)], axis=1)
+    return std, C, F.reshape(m, k, m, k), np.sqrt(np.maximum(spec, 0.0))
+
+
+def _block_covariance(A, free, simplex_rows):
+    n, k, _ = A.shape
+    B = np.zeros((n, k, k))
+    ok = np.ones(n, dtype=bool)
+    for c in range(n):
+        idx = np.flatnonzero(free[c])
+        if idx.size:
+            Bi = _inverse(A[c][np.ix_(idx, idx)])
+            if Bi is None:
+                ok[c] = False
+            else:
+                B[c][np.ix_(idx, idx)] = Bi
+    C = B.copy()
+    if simplex_rows is not None:
+        in_S = np.zeros(n, dtype=bool)
+        in_S[np.asarray(simplex_rows, dtype=np.int64)] = True
+        sel = in_S & ok
+        M = B[sel].sum(0)
+        act = np.flatnonzero(np.diag(M) > 0)            # columns with a free entry
+        if act.size:
+            Ba = B[sel][:, :, act]                       # (s, k, r)
+            C[sel] -= Ba @ np.linalg.solve(M[np.ix_(act, act)], np.swapaxes(Ba, 1, 2))
+            C[sel] = 0.5 * (C[sel] + np.swapaxes(C[sel], 1, 2))
+    C[~ok] = np.nan
+    std = np.sqrt(np.maximum(np.diagonal(C, axis1=1, axis2=2), 0.0))
+    std[~ok] = np.nan
+    return std, C, A, std.copy()

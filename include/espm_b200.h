@@ -189,8 +189,8 @@ typedef struct espm_state {
     void* W_next;
     const void* GW_cur;     /* n_pad x kp */
     const void* GWc_cur;    /* max(GW, ls), n_pad x kp (written by every espm_gw_prepare; read by the X passes only with
-                             * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats and
-                             * espm_abundance_info) */
+                             * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats,
+                             * espm_abundance_info and espm_phase_info) */
     void* GW_next;
     void* GWc_next;
     void* gwstats_cur;      /* 2*kp (c dtype): colsum(GW), colsum(max(GW,ls)) over the n real rows */
@@ -380,6 +380,19 @@ int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out,
  * order: two calls give identical bits, and a pixel shard gives the bits of the whole image.  Two launches.
  */
 int espm_abundance_info(const espm_state* st, int simplex, double* out, void* stream);
+/*
+ * Poisson information of the phases, per channel, over this rank's pixels (SmoothNMF.phase_uncertainty), one pass over
+ * Xt in W-pass order:
+ *   y_cj      = sum_a g_ca h_aj,   g = max(GW, ls), h = max(H, ls)           (the clamped Y of the KL loss)
+ *   A_c[a,b]  = sum_j x_cj h_aj h_bj / y_cj^2
+ * The information of vec(W) is F[(e,a),(f,b)] = sum_c G_ce G_cf A_c[a,b].
+ * out: [k (k + 1) / 2][n] doubles, A_c as its packed upper triangle row by row ((0,0), (0,1), ..., (1,1), ...).
+ * scratch: espm_phase_info_scratch bytes (a tile-major copy of max(H, ls) and the per-CTA channel sums).
+ * Reads Xt, GWc_cur, H_cur (k x ldh) and log_shift; writes no record and no device flag.  No atomics, fixed summation
+ * order: two calls give identical bits.  Three launches.
+ */
+int espm_phase_info_scratch(const espm_state* st, int64_t* bytes_out);
+int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stream);
 /*
  * Per-pixel assembly (updates.py:132-142): num, den with the log and Laplacian surrogates, the loss
  * regularisers of the CURRENT iterate (measures.py:548,577), rel_H (base.py:324), and either
