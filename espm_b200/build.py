@@ -18,13 +18,10 @@ OBJDIR = os.path.join(LIBDIR, "obj")
 LIBNAME = "libespm_b200.so"
 LIBPATH = os.path.join(LIBDIR, LIBNAME)
 
-SOURCES = ["api.cu", "xpass_f32f32.cu", "xpass_f32f64.cu", "xpass_f64f64.cu", "xpass_u8f32.cu", "xpass_u16f32.cu",
-           "small_f32.cu", "small_f64.cu", "ingest.cu", "fitstats_f32.cu", "fitstats_f64.cu",
-           "hinfo_f32.cu", "hinfo_f64.cu", "winfo_f32.cu", "winfo_f64.cu"]
+SOURCES = ["api.cu", "stream_f32f32.cu", "stream_f32f64.cu", "stream_f64f64.cu", "stream_u8f32.cu", "stream_u16f32.cu",
+           "small_f32.cu", "small_f64.cu", "ingest.cu"]
 HEADERS = ["common.cuh", "xpass.cuh", "xpass_inst.cuh", "small.cuh", "small_inst.cuh", "ingest.cuh", "ingest_decl.h",
-           "fitstats.cuh", "fitstats_decl.h", "hinfo.cuh", "hinfo_decl.h",
-           "winfo.cuh", "winfo_decl.h",
-           os.path.join("..", "..", "include", "espm_b200.h")]
+           "fitstats.cuh", "hinfo.cuh", "winfo.cuh", os.path.join("..", "..", "include", "espm_b200.h")]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = [

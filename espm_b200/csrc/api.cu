@@ -6,11 +6,8 @@
 #include <cstdio>
 #include <cstring>
 
-#include "fitstats_decl.h"
-#include "hinfo_decl.h"
 #include "ingest_decl.h"
 #include "small_inst.cuh"
-#include "winfo_decl.h"
 #include "xpass_inst.cuh"
 
 namespace espm {
@@ -31,23 +28,16 @@ static int pad_k(int k) {
     return -1;
 }
 
-typedef int (*xpass_fn)(const XPassLaunch&, const XPassArgs*, int*, cudaStream_t);
+static const StreamPair* const stream_pairs[] = {&stream_f32f32, &stream_f32f64, &stream_f64f64, &stream_u8f32,
+                                                  &stream_u16f32};
 
-static xpass_fn pick_xpass(const espm_state* st) {
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return xpass_f32f32;
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return xpass_f32f64;
-    if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) return xpass_f64f64;
-    if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) return xpass_u8f32;
-    if (st->x_dtype == ESPM_U16 && st->c_dtype == ESPM_F32) return xpass_u16f32;
+// the launchers of the state's (storage, compute) pair; null, with the error set, for a pair without kernels
+static const StreamPair* stream_pair(const espm_state* st) {
+    for (const StreamPair* row : stream_pairs)
+        if (row->x_dtype == st->x_dtype && row->c_dtype == st->c_dtype) return row;
+    set_error("unsupported dtype pair x=%d c=%d (f64 storage requires f64 arithmetic, uint8 / uint16 storage fp32)",
+              st->x_dtype, st->c_dtype);
     return nullptr;
-}
-
-static int sizes_of(const espm_state* st, int safe, XPassSizes* o) {
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return xpass_sizes<float, float>(st->kp, safe, o);
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return xpass_sizes<float, double>(st->kp, safe, o);
-    if (st->x_dtype == ESPM_U8) return xpass_sizes<uint8_t, float>(st->kp, safe, o);
-    if (st->x_dtype == ESPM_U16) return xpass_sizes<uint16_t, float>(st->kp, safe, o);
-    return xpass_sizes<double, double>(st->kp, safe, o);
 }
 
 // the Frobenius branches never divide by G W H and their loss does not clamp (measures.py:350-385)
@@ -65,11 +55,7 @@ static int check_state(const espm_state* st) {
         set_error("null state");
         return ESPM_ERR_BAD_ARG;
     }
-    if (!pick_xpass(st)) {
-        set_error("unsupported dtype pair x=%d c=%d (f64 storage requires f64 arithmetic, uint8 / uint16 storage fp32)",
-                  st->x_dtype, st->c_dtype);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    if (!stream_pair(st)) return ESPM_ERR_UNSUPPORTED;
     if (st->k < 1 || st->k > ESPM_MAX_K) {
         set_error("n_components=%d is outside the supported range 1..%d", st->k, ESPM_MAX_K);
         return ESPM_ERR_UNSUPPORTED;
@@ -191,32 +177,24 @@ int espm_plan(espm_state* st) {
 
     // The plan is made for the SAFE variant's shared-memory footprint so that switching on the
     // clamp / dual-loss fallbacks mid-fit never needs a re-plan.
+    const StreamPair* row = stream_pair(st);
     XPassSizes z;
-    rc = sizes_of(st, 1, &z);
+    rc = row->xpass_sizes(st->kp, 1, &z);
     if (rc) return rc;
     st->cs = z.cs;
     st->n_pad = (st->n + 31) / 32 * 32;   // whole stages for every storage type (CS is 32 or 16)
     const int NS = st->n_pad / z.cs;
-    const int smem_cap = (int)prop.sharedMemPerBlockOptin;                      // 227 KiB on B200
-    auto budget_for = [&](int want_occ) {
-        const int per_cta = (int)(prop.sharedMemPerMultiprocessor / want_occ) - 1024;  // 1 KiB reserved per CTA
-        return per_cta < smem_cap ? per_cta : smem_cap;
-    };
-    xpass_fn fn = pick_xpass(st);
+    const SmemLimits lim{(int)prop.sharedMemPerMultiprocessor, (int)prop.sharedMemPerBlockOptin};   // 228, 227 KiB on B200
 
     // ---- H pass ----
-    int depth = (budget_for(z.h_occ) - z.fixed - z.h_tail) / z.h_stride;
-    if (depth > 8) depth = 8;
-    if (depth < 2) {
-        set_error("shared memory budget too small for the H pass (kp=%d)", st->kp);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    const int depth = ring_depth(lim, z.h_occ, z.fixed, z.h_tail, z.h_stride, 8, "H pass", st->kp);
+    if (depth < 0) return depth;
     st->h_depth = depth;
     st->h_smem = z.fixed + depth * z.h_stride + z.h_tail;
     int occ = 0;
     {
         XPassLaunch l{XPASS_H, st->kp, 1, 1, st->h_smem, XMODE_KL};
-        rc = fn(l, nullptr, &occ, 0);
+        rc = row->xpass(l, nullptr, &occ, 0);
         if (rc) return rc;
         if (occ < 1) {
             set_error("H pass kernel does not fit on an SM (smem=%d)", st->h_smem);
@@ -249,46 +227,33 @@ int espm_plan(espm_state* st) {
 
     // ---- W pass: contiguous ranges of (channel block, tile) units, one per CTA ----
     {
-        int wdepth = (budget_for(z.w_occ) - z.fixed - z.w_tail) / z.w_stride;
-        if (wdepth > 8) wdepth = 8;
         // Measured on B200 (C3 f32, profiles/r01f_summary.md): the W pass is FASTER with a shallow ring -- 6 stages
         // 0.347 ms, 5: 0.340, 4: 0.323, 3: 0.316, 2: 0.344.  Consecutive units of a CTA are 1 MiB apart in Xt (same
         // channel block, next tile), so every stage in flight opens another DRAM page; three stages per CTA keep the
         // HBM queues short enough for the 592 concurrent streams.
-        if (wdepth > 3) wdepth = 3;
-        if (wdepth < 2) {
-            set_error("shared memory budget too small for the W pass (kp=%d)", st->kp);
-            return ESPM_ERR_UNSUPPORTED;
-        }
+        const int wdepth = ring_depth(lim, z.w_occ, z.fixed, z.w_tail, z.w_stride, 3, "W pass", st->kp);
+        if (wdepth < 0) return wdepth;
         st->w_depth = wdepth;
         st->w_smem = z.fixed + wdepth * z.w_stride + z.w_tail;
         int wocc = 0;
         XPassLaunch l{XPASS_W, st->kp, 1, 1, st->w_smem, XMODE_KL};
-        rc = fn(l, nullptr, &wocc, 0);
+        rc = row->xpass(l, nullptr, &wocc, 0);
         if (rc) return rc;
         if (wocc < 1) {
             set_error("W pass kernel does not fit on an SM (smem=%d)", st->w_smem);
             return ESPM_ERR_UNSUPPORTED;
         }
-        const long long total = (long long)NS * st->n_tiles;
-        const long long cap_w = (long long)st->n_sms * wocc;
-        const long long upc = (total + cap_w - 1) / cap_w;
-        st->w_upc = (int)upc;
-        st->w_grid = (int)((total + upc - 1) / upc);
-        int nr = 1;
-        for (int cb = 0; cb < NS; ++cb) {
-            const int c = w_last_cta(cb, st->n_tiles, st->w_upc) - w_first_cta(cb, st->n_tiles, st->w_upc) + 1;
-            if (c > nr) nr = c;
-        }
-        st->w_nr = nr;
+        plan_w_units(NS, st->n_tiles, (long long)st->n_sms * wocc, &st->w_upc, &st->w_grid, &st->w_nr);
     }
     return ESPM_OK;
 }
 
 int espm_plan_info(const espm_state* st, int32_t* info8) {
     if (!st || !info8) return ESPM_ERR_BAD_ARG;
+    const StreamPair* row = stream_pair(st);
+    if (!row) return ESPM_ERR_UNSUPPORTED;
     XPassSizes z;
-    int rc = sizes_of(st, 1, &z);
+    int rc = row->xpass_sizes(st->kp, 1, &z);
     if (rc) return rc;
     info8[0] = z.h_stride;
     info8[1] = z.w_stride;
@@ -427,17 +392,7 @@ int espm_h_pass(const espm_state* st, void* stream) {
     // (the kernel also clears the trace mask of the coming h_finish)
     XPassArgs a = make_args(st, false);
     XPassLaunch l{XPASS_H, st->kp, is_safe(st) ? 1 : 0, st->h_grid, st->h_smem, h_mode(st)};
-    return pick_xpass(st)(l, &a, nullptr, (cudaStream_t)stream);
-}
-
-typedef int (*fit_stats_fn)(const espm_state*, double*, double*, void*, int64_t*, cudaStream_t);
-
-static fit_stats_fn pick_fit_stats(const espm_state* st) {
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return fit_stats_f32f32;
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return fit_stats_f32f64;
-    if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) return fit_stats_f64f64;
-    if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) return fit_stats_u8f32;
-    return fit_stats_u16f32;   // check_state rejected every other pair
+    return stream_pair(st)->xpass(l, &a, nullptr, (cudaStream_t)stream);
 }
 
 int espm_fit_stats_scratch(const espm_state* st, int64_t* bytes_out) {
@@ -447,7 +402,7 @@ int espm_fit_stats_scratch(const espm_state* st, int64_t* bytes_out) {
         set_error("espm_fit_stats_scratch: null output");
         return ESPM_ERR_BAD_ARG;
     }
-    return pick_fit_stats(st)(st, nullptr, nullptr, nullptr, bytes_out, nullptr);
+    return stream_pair(st)->fit_stats(st, nullptr, nullptr, nullptr, bytes_out, nullptr);
 }
 
 int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out, void* scratch, void* stream) {
@@ -457,10 +412,8 @@ int espm_fit_stats(const espm_state* st, double* pixel_out, double* channel_out,
         set_error("espm_fit_stats: null output, scratch or input buffer");
         return ESPM_ERR_BAD_ARG;
     }
-    return pick_fit_stats(st)(st, pixel_out, channel_out, scratch, nullptr, (cudaStream_t)stream);
+    return stream_pair(st)->fit_stats(st, pixel_out, channel_out, scratch, nullptr, (cudaStream_t)stream);
 }
-
-typedef int (*h_info_fn)(const espm_state*, int, double*, cudaStream_t);
 
 int espm_abundance_info(const espm_state* st, int simplex, double* out, void* stream) {
     int rc = check_state(st);
@@ -469,22 +422,7 @@ int espm_abundance_info(const espm_state* st, int simplex, double* out, void* st
         set_error("espm_abundance_info: null output or input buffer");
         return ESPM_ERR_BAD_ARG;
     }
-    h_info_fn fn = h_info_u16f32;   // check_state rejected every other pair
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) fn = h_info_f32f32;
-    else if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) fn = h_info_f32f64;
-    else if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) fn = h_info_f64f64;
-    else if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) fn = h_info_u8f32;
-    return fn(st, simplex ? 1 : 0, out, (cudaStream_t)stream);
-}
-
-typedef int (*w_info_fn)(const espm_state*, double*, void*, int64_t*, cudaStream_t);
-
-static w_info_fn pick_w_info(const espm_state* st) {
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F32) return w_info_f32f32;
-    if (st->x_dtype == ESPM_F32 && st->c_dtype == ESPM_F64) return w_info_f32f64;
-    if (st->x_dtype == ESPM_F64 && st->c_dtype == ESPM_F64) return w_info_f64f64;
-    if (st->x_dtype == ESPM_U8 && st->c_dtype == ESPM_F32) return w_info_u8f32;
-    return w_info_u16f32;   // check_state rejected every other pair
+    return stream_pair(st)->h_info(st, simplex ? 1 : 0, out, (cudaStream_t)stream);
 }
 
 int espm_phase_info_scratch(const espm_state* st, int64_t* bytes_out) {
@@ -494,7 +432,7 @@ int espm_phase_info_scratch(const espm_state* st, int64_t* bytes_out) {
         set_error("espm_phase_info_scratch: null output");
         return ESPM_ERR_BAD_ARG;
     }
-    return pick_w_info(st)(st, nullptr, nullptr, bytes_out, nullptr);
+    return stream_pair(st)->w_info(st, nullptr, nullptr, bytes_out, nullptr);
 }
 
 int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stream) {
@@ -504,7 +442,7 @@ int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stre
         set_error("espm_phase_info: null output, scratch or input buffer");
         return ESPM_ERR_BAD_ARG;
     }
-    return pick_w_info(st)(st, out, scratch, nullptr, (cudaStream_t)stream);
+    return stream_pair(st)->w_info(st, out, scratch, nullptr, (cudaStream_t)stream);
 }
 
 int espm_w_pass(const espm_state* st, void* stream) {
@@ -512,7 +450,7 @@ int espm_w_pass(const espm_state* st, void* stream) {
     if (rc) return rc;
     XPassArgs a = make_args(st, true);
     XPassLaunch l{XPASS_W, st->kp, is_safe(st) ? 1 : 0, st->w_grid, st->w_smem, w_mode(st)};
-    return pick_xpass(st)(l, &a, nullptr, (cudaStream_t)stream);
+    return stream_pair(st)->xpass(l, &a, nullptr, (cudaStream_t)stream);
 }
 
 static void loop_bind(espm_state* st, const espm_loop* lp) {

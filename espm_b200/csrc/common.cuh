@@ -35,6 +35,23 @@ void set_error(const char* fmt, ...);
         }                                                                                   \
     } while (0)
 
+// Runs the statement with `constexpr int KP` set to the padded component count kp (one instance per supported width);
+// any other kp is an error.  Variadic so that the statement may hold template argument lists.
+#define ESPM_KP_SWITCH(kp, ...)                                         \
+    switch (kp) {                                                       \
+        case 2: { constexpr int KP = 2; __VA_ARGS__; break; }           \
+        case 3: { constexpr int KP = 3; __VA_ARGS__; break; }           \
+        case 4: { constexpr int KP = 4; __VA_ARGS__; break; }           \
+        case 5: { constexpr int KP = 5; __VA_ARGS__; break; }           \
+        case 6: { constexpr int KP = 6; __VA_ARGS__; break; }           \
+        case 8: { constexpr int KP = 8; __VA_ARGS__; break; }           \
+        case 12: { constexpr int KP = 12; __VA_ARGS__; break; }         \
+        case 16: { constexpr int KP = 16; __VA_ARGS__; break; }         \
+        default:                                                        \
+            set_error("unsupported padded component count kp=%d", kp);  \
+            return ESPM_ERR_BAD_ARG;                                    \
+    }
+
 // ---------------------------------------------------------------- mbarrier / bulk-copy PTX
 __device__ __forceinline__ uint32_t smem_u32(const void* p) {
     return static_cast<uint32_t>(__cvta_generic_to_shared(p));

@@ -6,9 +6,8 @@
 //
 // and their sums over channels (per pixel) and over pixels (per channel), together with those of x and y.
 //
-// Same work distribution and pipeline as the H pass (xpass.cuh): one producer warp fills a ring of stages with TMA
-// bulk copies of one (tile, CS-channel chunk) of Xt plus the matching rows of the clamped GW (GWc_cur, written by
-// espm_gw_prepare); a lane owns PPL pixels of the tile and walks the channels of its warp slot.  So
+// The stages come from produce_tile_stages (xpass.cuh) with the clamped GW (GWc_cur, written by espm_gw_prepare);
+// a lane owns PPL pixels of the tile and walks the channels of its warp slot.  So
 //   - the per-pixel sums stay in the lane across the stages of a tile (terms of one stage are added in the compute
 //     type, then into fp64 accumulators), and the NSLOT warps that share a pixel are added in fp64, in slot order,
 //     through shared memory once per tile;
@@ -98,17 +97,8 @@ __global__ void __launch_bounds__(XPASS_THREADS, 1) fit_stats_kernel(const FitSt
             const uint64_t pol_x = l2_policy_evict_first();
             const uint64_t pol_gw = l2_policy_evict_last();
             typename Ring<F::STRIDE>::Pos pos{0, 0u};
-            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
-                for (int st = 0; st < NS; ++st, ring.next(pos)) {
-                    ring.acquire(pos);
-                    unsigned char* sp = ring.stage(pos.slot);
-                    mbar_expect_tx(&ring.full[pos.slot], G::X_BYTES + F::S::GW_BYTES);
-                    const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)st * G::CS) * TILE_PX;
-                    tma_bulk_g2s(sp, xsrc, G::X_BYTES, &ring.full[pos.slot], pol_x);
-                    const TC* gsrc = reinterpret_cast<const TC*>(a.GWc) + (size_t)st * G::CS * KP;
-                    tma_bulk_g2s(sp + G::X_BYTES, gsrc, F::S::GW_BYTES, &ring.full[pos.slot], pol_gw);
-                }
-            }
+            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x)
+                produce_tile_stages<TX, TC, KP, &FitStatsArgs::GWc>(ring, pos, pol_x, pol_gw, a, tile, 0, NS, false);
         }
         return;
     }
@@ -301,23 +291,14 @@ static int fit_stats_do(const espm_state* st, double* pixel_out, double* channel
     // One CTA per SM with the deepest ring the shared memory holds (at most 8 stages, 128 KiB of X in flight per SM):
     // the kernel needs more registers than the 96 per thread of two CTAs per SM, and one CTA of 8 consumer warps has
     // 16 independent elements per lane and stage to hide the MUFU latency.
-    int dev = 0, optin = 0;
-    ESPM_CUDA_CHECK(cudaGetDevice(&dev));
-    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    int depth = (optin - F::FIXED - F::TAIL) / F::STRIDE;
-    if (depth > 8) depth = 8;
-    if (depth < 2) {
-        set_error("shared memory budget too small for the fit statistics kernel (kp=%d)", st->kp);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    SmemLimits lim;
+    int rc = query_smem_limits(&lim);
+    if (rc) return rc;
+    const int depth = ring_depth(lim, 1, F::FIXED, F::TAIL, F::STRIDE, 8, "fit statistics kernel", st->kp);
+    if (depth < 0) return depth;
     const int smem = F::FIXED + depth * F::STRIDE + F::TAIL;
-    ESPM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int occ = 0;
-    ESPM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, XPASS_THREADS, smem));
-    if (occ < 1) {
-        set_error("fit statistics kernel does not fit on an SM (smem=%d)", smem);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    if ((rc = kernel_fit(kern, smem, "fit statistics kernel", &occ))) return rc;
     const int cap = st->n_sms * occ;
     const int grid = st->n_tiles < cap ? st->n_tiles : cap;
     const int n_slots = grid * G::HALVES;
@@ -351,19 +332,7 @@ static int fit_stats_do(const espm_state* st, double* pixel_out, double* channel
 template <typename TX, typename TC>
 static int fit_stats_entry(const espm_state* st, double* pixel_out, double* channel_out, void* scratch,
                            int64_t* bytes_out, cudaStream_t stream) {
-    switch (st->kp) {
-        case 2: return fit_stats_do<TX, TC, 2>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 3: return fit_stats_do<TX, TC, 3>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 4: return fit_stats_do<TX, TC, 4>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 5: return fit_stats_do<TX, TC, 5>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 6: return fit_stats_do<TX, TC, 6>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 8: return fit_stats_do<TX, TC, 8>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 12: return fit_stats_do<TX, TC, 12>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        case 16: return fit_stats_do<TX, TC, 16>(st, pixel_out, channel_out, scratch, bytes_out, stream);
-        default:
-            set_error("unsupported padded component count kp=%d", st->kp);
-            return ESPM_ERR_BAD_ARG;
-    }
+    ESPM_KP_SWITCH(st->kp, return fit_stats_do<TX, TC, KP>(st, pixel_out, channel_out, scratch, bytes_out, stream));
 }
 
 }  // namespace espm

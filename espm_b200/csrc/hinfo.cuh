@@ -4,8 +4,7 @@
 //   y[c][j]    = sum_a g[c][a] h[a][j],   g = max(GW, ls), h = max(H, ls)      (the Y of KLdiv_loss, measures.py:493-497)
 //   F_j[a][b]  = sum_c x[c][j] g[c][a] g[c][b] / y[c][j]^2                     (Hessian of the KL loss in H[:, j])
 //
-// h_info_kernel streams Xt once with the work distribution and pipeline of the H pass (xpass.cuh): one producer warp
-// fills a ring of stages with TMA bulk copies of one (tile, CS-channel chunk) of Xt plus the matching rows of GWc_cur; a
+// h_info_kernel streams Xt once in H pass order, the stages coming from produce_tile_stages (xpass.cuh) with GWc_cur; a
 // lane owns PPL pixels of the tile and walks the channels of its warp slot.  Per element: y (KP FMA), one reciprocal r,
 // w = x r r, u_a = w g_a (KP multiplies) and the KP (KP + 1) / 2 FMAs u_a g_b of the upper triangle.  fp32: packed
 // f32x2 arithmetic, one MUFU.RCP per element (the H pass spends two); fp64: the Newton reciprocal of Num<double>, no log.
@@ -93,17 +92,8 @@ __global__ void __launch_bounds__(XPASS_THREADS, (HInfoGeom<TX, TC, KP>::OCC)) h
             const uint64_t pol_x = l2_policy_evict_first();
             const uint64_t pol_gw = l2_policy_evict_last();
             typename Ring<I::STRIDE>::Pos pos{0, 0u};
-            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x) {
-                for (int st = 0; st < NS; ++st, ring.next(pos)) {
-                    ring.acquire(pos);
-                    unsigned char* sp = ring.stage(pos.slot);
-                    mbar_expect_tx(&ring.full[pos.slot], I::X_BYTES + I::S::GW_BYTES);
-                    const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)st * I::CS) * TILE_PX;
-                    tma_bulk_g2s(sp, xsrc, I::X_BYTES, &ring.full[pos.slot], pol_x);
-                    const TC* gsrc = reinterpret_cast<const TC*>(a.GWc) + (size_t)st * I::CS * KP;
-                    tma_bulk_g2s(sp + I::X_BYTES, gsrc, I::S::GW_BYTES, &ring.full[pos.slot], pol_gw);
-                }
-            }
+            for (int tile = blockIdx.x; tile < a.n_tiles; tile += gridDim.x)
+                produce_tile_stages<TX, TC, KP, &HInfoArgs::GWc>(ring, pos, pol_x, pol_gw, a, tile, 0, NS, false);
         }
         return;
     }
@@ -321,26 +311,14 @@ template <typename TX, typename TC, int KP>
 static int h_info_do(const espm_state* st, int simplex, double* out, cudaStream_t stream) {
     using I = HInfoGeom<TX, TC, KP>;
     void (*kern)(const HInfoArgs) = h_info_kernel<TX, TC, KP>;
-    int dev = 0, optin = 0, per_sm = 0;
-    ESPM_CUDA_CHECK(cudaGetDevice(&dev));
-    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
-    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
-    int budget = per_sm / I::OCC - 1024;   // 1 KiB reserved per CTA
-    if (budget > optin) budget = optin;
-    int depth = (budget - I::FIXED - I::TAIL) / I::STRIDE;
-    if (depth > 8) depth = 8;
-    if (depth < 2) {
-        set_error("shared memory budget too small for the abundance information kernel (kp=%d)", st->kp);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    SmemLimits lim;
+    int rc = query_smem_limits(&lim);
+    if (rc) return rc;
+    const int depth = ring_depth(lim, I::OCC, I::FIXED, I::TAIL, I::STRIDE, 8, "abundance information kernel", st->kp);
+    if (depth < 0) return depth;
     const int smem = I::FIXED + depth * I::STRIDE + I::TAIL;
-    ESPM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int occ = 0;
-    ESPM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, XPASS_THREADS, smem));
-    if (occ < 1) {
-        set_error("abundance information kernel does not fit on an SM (smem=%d)", smem);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    if ((rc = kernel_fit(kern, smem, "abundance information kernel", &occ))) return rc;
     const int cap = st->n_sms * occ;
     const int grid = st->n_tiles < cap ? st->n_tiles : cap;
     const int k = st->k, p = st->p_loc;
@@ -367,19 +345,7 @@ static int h_info_do(const espm_state* st, int simplex, double* out, cudaStream_
 
 template <typename TX, typename TC>
 static int h_info_entry(const espm_state* st, int simplex, double* out, cudaStream_t stream) {
-    switch (st->kp) {
-        case 2: return h_info_do<TX, TC, 2>(st, simplex, out, stream);
-        case 3: return h_info_do<TX, TC, 3>(st, simplex, out, stream);
-        case 4: return h_info_do<TX, TC, 4>(st, simplex, out, stream);
-        case 5: return h_info_do<TX, TC, 5>(st, simplex, out, stream);
-        case 6: return h_info_do<TX, TC, 6>(st, simplex, out, stream);
-        case 8: return h_info_do<TX, TC, 8>(st, simplex, out, stream);
-        case 12: return h_info_do<TX, TC, 12>(st, simplex, out, stream);
-        case 16: return h_info_do<TX, TC, 16>(st, simplex, out, stream);
-        default:
-            set_error("unsupported padded component count kp=%d", st->kp);
-            return ESPM_ERR_BAD_ARG;
-    }
+    ESPM_KP_SWITCH(st->kp, return h_info_do<TX, TC, KP>(st, simplex, out, stream));
 }
 
 }  // namespace espm

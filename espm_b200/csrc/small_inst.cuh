@@ -29,21 +29,6 @@ struct DichoArgs {
     int* its_out;
 };
 
-#define ESPM_KP_SWITCH(kp, STMT)                                         \
-    switch (kp) {                                                        \
-        case 2: { constexpr int KP = 2; STMT; break; }                   \
-        case 3: { constexpr int KP = 3; STMT; break; }                   \
-        case 4: { constexpr int KP = 4; STMT; break; }                   \
-        case 5: { constexpr int KP = 5; STMT; break; }                   \
-        case 6: { constexpr int KP = 6; STMT; break; }                   \
-        case 8: { constexpr int KP = 8; STMT; break; }                   \
-        case 12: { constexpr int KP = 12; STMT; break; }                 \
-        case 16: { constexpr int KP = 16; STMT; break; }                 \
-        default:                                                         \
-            set_error("unsupported padded component count kp=%d", kp);   \
-            return ESPM_ERR_BAD_ARG;                                     \
-    }
-
 template <typename TC>
 static int small_launch_t(int op, const espm_state* st, cudaStream_t s) {
     const int kp = st->kp;

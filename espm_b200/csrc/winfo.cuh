@@ -8,10 +8,8 @@
 // Three launches:
 //   w_info_tiles_kernel  Ht[tile][KP][128] = max(H_cur, ls) tile-major in the caller's scratch (rows >= k are 0, pad
 //                        pixels hold ls, so y > 0 there and their x = 0 gives w = x r r = 0);
-//   w_info_kernel        the sums, with the work layout of the W pass (xpass.cuh): units (channel block, tile) ordered
-//                        channel-block major, CTA i owns the contiguous range [i upc, (i + 1) upc); one producer warp
-//                        copies the X chunk and the H tile of a unit into a ring stage (two TMA bulk copies); the GW
-//                        rows of the channel block sit in shared memory while the block is processed;
+//   w_info_kernel        the sums, in W pass order: the stages come from produce_units (xpass.cuh); the GW rows of the
+//                        channel block sit in shared memory while the block is processed;
 //   w_info_fold_kernel   A[tri(a, b)][c] = sum of the CTA slots of channel c, in slot order.
 //
 // Work of a lane: PPL pixels of the tile (HALVES warps cover a 128-px row) x CPW channels (warp slot s owns channels
@@ -41,7 +39,7 @@ struct WInfoArgs {
     const void* GWc;      // [n_pad][KP], max(GW, ls) on the real entries
     const void* Ht;       // [n_tiles][KP][TILE_PX], written by w_info_tiles_kernel
     double* part;         // [nr][n_pad][NT] CTA slots
-    int n_pad, k, n_tiles, nstages_tile, upc, depth;
+    int n_pad, k, n_tiles, nstages_tile, w_upc, depth;
 };
 
 template <typename TX, typename TC, int KP>
@@ -87,11 +85,8 @@ __global__ void __launch_bounds__(XPASS_THREADS, 1) w_info_kernel(const WInfoArg
     double* acc64 = reinterpret_cast<double*>(tail0 + I::GW_BYTES);                // [HALVES][CS][NT]
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long total = (long long)a.nstages_tile * a.n_tiles;
-    const long long u0 = (long long)blockIdx.x * a.upc;
-    const long long u1 = (u0 + a.upc < total) ? u0 + a.upc : total;
-    const int n_units = (u1 > u0) ? (int)(u1 - u0) : 0;
-    const int cb0 = (int)(u0 / a.n_tiles), tile0 = (int)(u0 - (long long)cb0 * a.n_tiles);
+    const UnitRange units(a);
+    const int n_units = units.n_units, cb0 = units.cb0, tile0 = units.tile0;
 
     if (threadIdx.x == 0) ring.init();
     for (int i = threadIdx.x; i < I::HALVES * I::CS * NT; i += blockDim.x) acc64[i] = 0.0;
@@ -99,23 +94,8 @@ __global__ void __launch_bounds__(XPASS_THREADS, 1) w_info_kernel(const WInfoArg
 
     if (warp == N_CONSUMER_WARPS) {
         if (lane == 0) {
-            const uint64_t pol_x = l2_policy_evict_first();
-            const uint64_t pol_h = l2_policy_evict_last();
-            const TC* Ht = reinterpret_cast<const TC*>(a.Ht);
             typename Ring<I::STRIDE>::Pos pos{0, 0u};
-            int cb = cb0, tile = tile0;
-            for (int i = 0; i < n_units; ++i, ring.next(pos)) {
-                ring.acquire(pos);
-                unsigned char* sp = ring.stage(pos.slot);
-                mbar_expect_tx(&ring.full[pos.slot], I::STRIDE);
-                const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)cb * I::CS) * TILE_PX;
-                tma_bulk_g2s(sp, xsrc, I::X_BYTES, &ring.full[pos.slot], pol_x);
-                tma_bulk_g2s(sp + I::X_BYTES, Ht + (size_t)tile * KP * TILE_PX, I::H_BYTES, &ring.full[pos.slot], pol_h);
-                if (++tile == a.n_tiles) {
-                    tile = 0;
-                    ++cb;
-                }
-            }
+            produce_units<TX, TC, KP, I::CS>(ring, pos, units, a);
         }
         return;
     }
@@ -159,7 +139,7 @@ __global__ void __launch_bounds__(XPASS_THREADS, 1) w_info_kernel(const WInfoArg
     // ends the channel block `cb` of this CTA: part[slot of this CTA in cb][channels of cb][NT]
     auto flush = [&](int cb) {
         named_bar_sync(1, N_CONSUMER_THREADS);
-        const int ps = blockIdx.x - w_first_cta(cb, a.n_tiles, a.upc);
+        const int ps = blockIdx.x - w_first_cta(cb, a.n_tiles, a.w_upc);
         double* out = a.part + ((size_t)ps * a.n_pad + (size_t)cb * I::CS) * NT;
         for (int i = threadIdx.x; i < I::CS * NT; i += N_CONSUMER_THREADS) {
             double v = acc64[i];
@@ -286,41 +266,26 @@ template <typename TX, typename TC, int KP>
 static int w_info_do(const espm_state* st, double* out, void* scratch, int64_t* bytes_out, cudaStream_t stream) {
     using I = WInfoGeom<TX, TC, KP>;
     void (*kern)(const WInfoArgs) = w_info_kernel<TX, TC, KP>;
-    int dev = 0, optin = 0;
-    ESPM_CUDA_CHECK(cudaGetDevice(&dev));
-    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    SmemLimits lim;
+    int rc = query_smem_limits(&lim);
+    if (rc) return rc;
     // about 96 KiB of X in flight per SM, the amount of the W pass's best ring (profiles/r01f_summary.md)
-    int depth = (optin - I::FIXED - I::TAIL) / I::STRIDE;
     const int want = 98304 / I::X_BYTES;
-    if (depth > want) depth = want;
-    if (depth > 8) depth = 8;
-    if (depth < 2) {
-        set_error("shared memory budget too small for the phase information kernel (kp=%d)", st->kp);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    const int depth = ring_depth(lim, 1, I::FIXED, I::TAIL, I::STRIDE, want < 8 ? want : 8, "phase information kernel",
+                                 st->kp);
+    if (depth < 0) return depth;
     const int smem = I::FIXED + depth * I::STRIDE + I::TAIL;
     const int NS = st->n_pad / I::CS;
-    const long long total = (long long)NS * st->n_tiles;
-    const long long upc = (total + st->n_sms - 1) / st->n_sms;
-    const int grid = (int)((total + upc - 1) / upc);
-    int nr = 1;
-    for (int cb = 0; cb < NS; ++cb) {
-        const int c = w_last_cta(cb, st->n_tiles, (int)upc) - w_first_cta(cb, st->n_tiles, (int)upc) + 1;
-        if (c > nr) nr = c;
-    }
+    int upc = 0, grid = 0, nr = 0;
+    plan_w_units(NS, st->n_tiles, st->n_sms, &upc, &grid, &nr);
     const size_t ht_bytes = ((size_t)st->n_tiles * I::H_BYTES + 255) / 256 * 256;
     const size_t part_bytes = (size_t)nr * st->n_pad * I::NT * sizeof(double);
     if (bytes_out) {
         *bytes_out = (int64_t)(ht_bytes + part_bytes);
         return ESPM_OK;
     }
-    ESPM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     int occ = 0;
-    ESPM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&occ, kern, XPASS_THREADS, smem));
-    if (occ < 1) {
-        set_error("phase information kernel does not fit on an SM (smem=%d)", smem);
-        return ESPM_ERR_UNSUPPORTED;
-    }
+    if ((rc = kernel_fit(kern, smem, "phase information kernel", &occ))) return rc;
     TC* Ht = reinterpret_cast<TC*>(scratch);
     const long long nh = (long long)KP * st->n_tiles * TILE_PX;
     w_info_tiles_kernel<TC, KP><<<(unsigned)((nh + 255) / 256), 256, 0, stream>>>(
@@ -335,11 +300,11 @@ static int w_info_do(const espm_state* st, double* out, void* scratch, int64_t* 
     a.k = st->k;
     a.n_tiles = st->n_tiles;
     a.nstages_tile = NS;
-    a.upc = (int)upc;
+    a.w_upc = upc;
     a.depth = depth;
     w_info_kernel<TX, TC, KP><<<grid, XPASS_THREADS, smem, stream>>>(a);
     ESPM_CUDA_CHECK(cudaGetLastError());
-    w_info_fold_kernel<KP><<<(st->n + 255) / 256, 256, 0, stream>>>(a.part, st->n_tiles, (int)upc, I::CS, st->n,
+    w_info_fold_kernel<KP><<<(st->n + 255) / 256, 256, 0, stream>>>(a.part, st->n_tiles, upc, I::CS, st->n,
                                                                     st->n_pad, st->k, out);
     ESPM_CUDA_CHECK(cudaGetLastError());
     return ESPM_OK;
@@ -347,19 +312,7 @@ static int w_info_do(const espm_state* st, double* out, void* scratch, int64_t* 
 
 template <typename TX, typename TC>
 static int w_info_entry(const espm_state* st, double* out, void* scratch, int64_t* bytes_out, cudaStream_t stream) {
-    switch (st->kp) {
-        case 2: return w_info_do<TX, TC, 2>(st, out, scratch, bytes_out, stream);
-        case 3: return w_info_do<TX, TC, 3>(st, out, scratch, bytes_out, stream);
-        case 4: return w_info_do<TX, TC, 4>(st, out, scratch, bytes_out, stream);
-        case 5: return w_info_do<TX, TC, 5>(st, out, scratch, bytes_out, stream);
-        case 6: return w_info_do<TX, TC, 6>(st, out, scratch, bytes_out, stream);
-        case 8: return w_info_do<TX, TC, 8>(st, out, scratch, bytes_out, stream);
-        case 12: return w_info_do<TX, TC, 12>(st, out, scratch, bytes_out, stream);
-        case 16: return w_info_do<TX, TC, 16>(st, out, scratch, bytes_out, stream);
-        default:
-            set_error("unsupported padded component count kp=%d", st->kp);
-            return ESPM_ERR_BAD_ARG;
-    }
+    ESPM_KP_SWITCH(st->kp, return w_info_do<TX, TC, KP>(st, out, scratch, bytes_out, stream));
 }
 
 }  // namespace espm

@@ -219,6 +219,76 @@ struct Ring {
 };
 
 // ------------------------------------------------------------------------------------------------
+// The two producers, called by the elected producer lane.  Every kernel that streams X uses one of them.  They read
+// Xt, n_pad (and Ht, n_tiles, w_upc) from the kernel's argument struct `a` where the copies are issued.  The kernel
+// owns the ring position `pos`: the H pass calls produce_tile_stages once per work item and continues the ring.  X is
+// copied with the evict-first L2 policy, the GW rows and H tiles, which every CTA reads, with evict-last.
+//
+// Tile stages (H pass order): the stages [s0, s1) of pixel tile `tile`, each the X chunk of CS channels plus the
+// CS x KP rows of a.*GW behind it; with `dual` (SAFE H pass only) also the rows of a.GWc at GW_BYTES_AL.
+// ------------------------------------------------------------------------------------------------
+template <typename TX, typename TC, int KP, auto GW, int STRIDE, typename Args>
+__device__ __forceinline__ void produce_tile_stages(Ring<STRIDE>& ring, typename Ring<STRIDE>::Pos& pos,
+                                                    uint64_t pol_x, uint64_t pol_gw, const Args& a, int tile, int s0,
+                                                    int s1, bool dual) {
+    using S = XPassSmem<TX, TC, KP, false>;
+    constexpr int CS = S::G::CS;
+    for (int st = s0; st < s1; ++st, ring.next(pos)) {
+        ring.acquire(pos);
+        const int slot = pos.slot;
+        unsigned char* sp = ring.stage(slot);
+        mbar_expect_tx(&ring.full[slot], S::X_BYTES + S::GW_BYTES * (dual ? 2 : 1));
+        const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)st * CS) * TILE_PX;
+        tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[slot], pol_x);
+        const TC* gsrc = reinterpret_cast<const TC*>(a.*GW) + (size_t)st * CS * KP;
+        tma_bulk_g2s(sp + S::X_BYTES, gsrc, S::GW_BYTES, &ring.full[slot], pol_gw);
+        if (dual) {
+            const TC* csrc = reinterpret_cast<const TC*>(a.GWc) + (size_t)st * CS * KP;
+            tma_bulk_g2s(sp + S::X_BYTES + S::GW_BYTES_AL, csrc, S::GW_BYTES, &ring.full[slot], pol_gw);
+        }
+    }
+}
+
+// Units (W pass order): work unit = (channel block of CS channels, pixel tile), ordered channel-block major; CTA i owns
+// the contiguous range [i w_upc, (i + 1) w_upc) of the nstages_tile x n_tiles units.
+struct UnitRange {
+    int n_units, cb0, tile0;
+    template <typename Args>
+    __device__ __forceinline__ explicit UnitRange(const Args& a) {
+        const long long total = (long long)a.nstages_tile * a.n_tiles;
+        const long long u0 = (long long)blockIdx.x * a.w_upc;
+        const long long u1 = (u0 + a.w_upc < total) ? u0 + a.w_upc : total;
+        n_units = (u1 > u0) ? (int)(u1 - u0) : 0;
+        cb0 = (int)(u0 / a.n_tiles);
+        tile0 = (int)(u0 - (long long)cb0 * a.n_tiles);
+    }
+};
+
+// One stage per unit: the X chunk of channel block cb of the tile, then the tile's KP x TILE_PX block of a.Ht.
+template <typename TX, typename TC, int KP, int CS, int STRIDE, typename Args>
+__device__ __forceinline__ void produce_units(Ring<STRIDE>& ring, typename Ring<STRIDE>::Pos& pos, const UnitRange& u,
+                                              const Args& a) {
+    constexpr int X_BYTES = CS * TILE_PX * (int)sizeof(TX);
+    constexpr int H_BYTES = KP * TILE_PX * (int)sizeof(TC);
+    const uint64_t pol_x = l2_policy_evict_first();
+    const uint64_t pol_h = l2_policy_evict_last();
+    const TC* Ht = reinterpret_cast<const TC*>(a.Ht);
+    int cb = u.cb0, tile = u.tile0;
+    for (int i = 0; i < u.n_units; ++i, ring.next(pos)) {
+        ring.acquire(pos);
+        unsigned char* sp = ring.stage(pos.slot);
+        mbar_expect_tx(&ring.full[pos.slot], X_BYTES + H_BYTES);
+        const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)cb * CS) * TILE_PX;
+        tma_bulk_g2s(sp, xsrc, X_BYTES, &ring.full[pos.slot], pol_x);
+        tma_bulk_g2s(sp + X_BYTES, Ht + (size_t)tile * KP * TILE_PX, H_BYTES, &ring.full[pos.slot], pol_h);
+        if (++tile == a.n_tiles) {
+            tile = 0;
+            ++cb;
+        }
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // H pass
 // ------------------------------------------------------------------------------------------------
 template <typename TX, typename TC, int KP, bool SAFE, int MODE = XMODE_KL>
@@ -253,25 +323,12 @@ h_pass_kernel(const XPassArgs a) {
         if (lane == 0) {
             const uint64_t pol_x = l2_policy_evict_first();
             const uint64_t pol_gw = l2_policy_evict_last();
-            const bool dual = SAFE && a.dual;
+            const bool dual = SAFE && a.dual;   // compile-time false in the non-SAFE instances
             typename Ring<S::H_STRIDE>::Pos pos{0, 0u};
             for (int it = blockIdx.x; it < n_items; it += gridDim.x) {
                 const int tile = it / a.nsplit, split = it - tile * a.nsplit;
                 const int s0 = (int)((long long)split * NS / a.nsplit), s1 = (int)((long long)(split + 1) * NS / a.nsplit);
-                for (int st = s0; st < s1; ++st, ring.next(pos)) {
-                    ring.acquire(pos);
-                    const int slot = pos.slot;
-                    unsigned char* sp = ring.stage(slot);
-                    mbar_expect_tx(&ring.full[slot], S::X_BYTES + S::GW_BYTES * (dual ? 2 : 1));
-                    const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)st * G::CS) * TILE_PX;
-                    tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[slot], pol_x);
-                    const TC* gsrc = reinterpret_cast<const TC*>(a.GW) + (size_t)st * G::CS * KP;
-                    tma_bulk_g2s(sp + S::X_BYTES, gsrc, S::GW_BYTES, &ring.full[slot], pol_gw);
-                    if (dual) {
-                        const TC* csrc = reinterpret_cast<const TC*>(a.GWc) + (size_t)st * G::CS * KP;
-                        tma_bulk_g2s(sp + S::X_BYTES + S::GW_BYTES_AL, csrc, S::GW_BYTES, &ring.full[slot], pol_gw);
-                    }
-                }
+                produce_tile_stages<TX, TC, KP, &XPassArgs::GW>(ring, pos, pol_x, pol_gw, a, tile, s0, s1, dual);
             }
         }
         return;
@@ -511,6 +568,63 @@ __host__ __device__ inline int w_last_cta(int cb, int n_tiles, int upc) {
     return (int)((((long long)cb + 1) * n_tiles - 1) / upc);
 }
 
+// ------------------------------------------------------------------------------------------------
+// Host planning shared by every X-streaming kernel.
+// ------------------------------------------------------------------------------------------------
+struct SmemLimits {
+    int per_sm, optin;   // shared memory per SM, and the opt-in maximum of one CTA
+};
+
+inline int query_smem_limits(SmemLimits* lim) {
+    int dev = 0;
+    ESPM_CUDA_CHECK(cudaGetDevice(&dev));
+    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&lim->optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev));
+    ESPM_CUDA_CHECK(cudaDeviceGetAttribute(&lim->per_sm, cudaDevAttrMaxSharedMemoryPerMultiprocessor, dev));
+    return ESPM_OK;
+}
+
+// Stages of `stride` bytes for a kernel compiled for `occ` CTAs per SM: the per-CTA budget is per_sm / occ less the
+// 1 KiB the runtime reserves per CTA, at most the opt-in maximum; `fixed` (barriers) and `tail` (epilogue) come first.
+// Returns the depth (at most max_depth), or a negative error code when fewer than two stages fit.
+inline int ring_depth(const SmemLimits& lim, int occ, int fixed, int tail, int stride, int max_depth, const char* what,
+                      int kp) {
+    int budget = lim.per_sm / occ - 1024;
+    if (budget > lim.optin) budget = lim.optin;
+    int depth = (budget - fixed - tail) / stride;
+    if (depth > max_depth) depth = max_depth;
+    if (depth < 2) {
+        set_error("shared memory budget too small for the %s (kp=%d)", what, kp);
+        return ESPM_ERR_UNSUPPORTED;
+    }
+    return depth;
+}
+
+// Sets the kernel's dynamic shared memory to `smem` and returns its resident CTAs per SM in *occ (>= 1).
+template <typename Kernel>
+inline int kernel_fit(Kernel kern, int smem, const char* what, int* occ) {
+    ESPM_CUDA_CHECK(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    ESPM_CUDA_CHECK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(occ, kern, XPASS_THREADS, smem));
+    if (*occ < 1) {
+        set_error("%s does not fit on an SM (smem=%d)", what, smem);
+        return ESPM_ERR_UNSUPPORTED;
+    }
+    return ESPM_OK;
+}
+
+// Splits the NS x n_tiles units of the W pass order over at most `cap` CTAs: units per CTA, CTAs, and the largest
+// number of CTAs that share a channel block (the partial slots per channel).
+inline void plan_w_units(int NS, int n_tiles, long long cap, int* upc, int* grid, int* nr) {
+    const long long total = (long long)NS * n_tiles;
+    const long long u = (total + cap - 1) / cap;
+    *upc = (int)u;
+    *grid = (int)((total + u - 1) / u);
+    *nr = 1;
+    for (int cb = 0; cb < NS; ++cb) {
+        const int c = w_last_cta(cb, n_tiles, *upc) - w_first_cta(cb, n_tiles, *upc) + 1;
+        if (c > *nr) *nr = c;
+    }
+}
+
 template <typename TX, typename TC, int KP, bool SAFE, int MODE = XMODE_KL>
 __global__ void __launch_bounds__(XPASS_THREADS, (XPassSmem<TX, TC, KP, SAFE>::W_OCC))
 w_pass_kernel(const XPassArgs a) {
@@ -529,11 +643,8 @@ w_pass_kernel(const XPassArgs a) {
     TC* tail = reinterpret_cast<TC*>(tail0 + S::GW_BYTES_AL);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const long long total = (long long)a.nstages_tile * a.n_tiles;
-    const long long u0 = (long long)blockIdx.x * a.w_upc;
-    const long long u1 = (u0 + a.w_upc < total) ? u0 + a.w_upc : total;
-    const int n_units = (u1 > u0) ? (int)(u1 - u0) : 0;
-    const int cb0 = (int)(u0 / a.n_tiles), tile0 = (int)(u0 - (long long)cb0 * a.n_tiles);
+    const UnitRange units(a);
+    const int n_units = units.n_units;
 
     if (threadIdx.x == 0) ring.init();      // shared memory only: may overlap the previous kernel's tail
     for (int i = threadIdx.x; i < G::HALVES * G::CS * KP; i += blockDim.x) tail[i] = TC(0);
@@ -543,24 +654,8 @@ w_pass_kernel(const XPassArgs a) {
 
     if (warp == N_CONSUMER_WARPS) {
         if (lane == 0) {
-            const uint64_t pol_x = l2_policy_evict_first();
-            const uint64_t pol_h = l2_policy_evict_last();
-            const TC* Ht = reinterpret_cast<const TC*>(a.Ht);
             typename Ring<S::W_STRIDE>::Pos pos{0, 0u};
-            int cb = cb0, tile = tile0;
-            for (int i = 0; i < n_units; ++i, ring.next(pos)) {
-                ring.acquire(pos);
-                unsigned char* sp = ring.stage(pos.slot);
-                mbar_expect_tx(&ring.full[pos.slot], S::X_BYTES + KP * S::HROW_BYTES);
-                const TX* xsrc = reinterpret_cast<const TX*>(a.Xt) + ((size_t)tile * a.n_pad + (size_t)cb * G::CS) * TILE_PX;
-                tma_bulk_g2s(sp, xsrc, S::X_BYTES, &ring.full[pos.slot], pol_x);
-                tma_bulk_g2s(sp + S::X_BYTES, Ht + (size_t)tile * KP * TILE_PX, KP * S::HROW_BYTES, &ring.full[pos.slot],
-                             pol_h);
-                if (++tile == a.n_tiles) {
-                    tile = 0;
-                    ++cb;
-                }
-            }
+            produce_units<TX, TC, KP, G::CS>(ring, pos, units, a);
         }
         return;
     }
@@ -624,7 +719,7 @@ w_pass_kernel(const XPassArgs a) {
     };
 
     typename Ring<S::W_STRIDE>::Pos pos{0, 0u};
-    int cb = cb0, tile = tile0;
+    int cb = units.cb0, tile = units.tile0;
     if (n_units > 0) load_gw(cb);
     for (int i = 0; i < n_units; ++i, ring.next(pos)) {
         ring.consumer_wait(pos);

@@ -1,5 +1,5 @@
-// Explicit instantiation helpers for the X-pass kernels: one translation unit per (storage, compute)
-// type pair so that the 48 template instances compile in parallel.
+// Host dispatch of the X-pass kernels, and the table row that bundles every X-streaming kernel family of one
+// (storage, compute) type pair.  Each pair is one translation unit (stream_<pair>.cu), so the pairs compile in parallel.
 #pragma once
 #include "xpass.cuh"
 
@@ -56,26 +56,14 @@ static int xpass_do(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cuda
     return ESPM_OK;
 }
 
-template <typename TX, typename TC, bool SAFE>
-static int xpass_by_kp(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream) {
-    switch (l.kp) {
-        case 2: return xpass_do<TX, TC, 2, SAFE>(l, a, occ_out, stream);
-        case 3: return xpass_do<TX, TC, 3, SAFE>(l, a, occ_out, stream);
-        case 4: return xpass_do<TX, TC, 4, SAFE>(l, a, occ_out, stream);
-        case 5: return xpass_do<TX, TC, 5, SAFE>(l, a, occ_out, stream);
-        case 6: return xpass_do<TX, TC, 6, SAFE>(l, a, occ_out, stream);
-        case 8: return xpass_do<TX, TC, 8, SAFE>(l, a, occ_out, stream);
-        case 12: return xpass_do<TX, TC, 12, SAFE>(l, a, occ_out, stream);
-        case 16: return xpass_do<TX, TC, 16, SAFE>(l, a, occ_out, stream);
-        default:
-            set_error("unsupported padded component count kp=%d", l.kp);
-            return ESPM_ERR_BAD_ARG;
-    }
-}
-
 template <typename TX, typename TC>
 static int xpass_entry(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream) {
-    return l.safe ? xpass_by_kp<TX, TC, true>(l, a, occ_out, stream) : xpass_by_kp<TX, TC, false>(l, a, occ_out, stream);
+    if (l.safe) {
+        ESPM_KP_SWITCH(l.kp, return xpass_do<TX, TC, KP, true>(l, a, occ_out, stream));
+    } else {
+        ESPM_KP_SWITCH(l.kp, return xpass_do<TX, TC, KP, false>(l, a, occ_out, stream));
+    }
+    return ESPM_OK;
 }
 
 // sizes needed by the planner (host)
@@ -104,25 +92,26 @@ static void xpass_sizes_kp(int safe, XPassSizes* o) {
 
 template <typename TX, typename TC>
 static int xpass_sizes(int kp, int safe, XPassSizes* o) {
-    switch (kp) {
-        case 2: xpass_sizes_kp<TX, TC, 2>(safe, o); return ESPM_OK;
-        case 3: xpass_sizes_kp<TX, TC, 3>(safe, o); return ESPM_OK;
-        case 4: xpass_sizes_kp<TX, TC, 4>(safe, o); return ESPM_OK;
-        case 5: xpass_sizes_kp<TX, TC, 5>(safe, o); return ESPM_OK;
-        case 6: xpass_sizes_kp<TX, TC, 6>(safe, o); return ESPM_OK;
-        case 8: xpass_sizes_kp<TX, TC, 8>(safe, o); return ESPM_OK;
-        case 12: xpass_sizes_kp<TX, TC, 12>(safe, o); return ESPM_OK;
-        case 16: xpass_sizes_kp<TX, TC, 16>(safe, o); return ESPM_OK;
-        default: set_error("unsupported padded component count kp=%d", kp); return ESPM_ERR_BAD_ARG;
-    }
+    ESPM_KP_SWITCH(kp, xpass_sizes_kp<TX, TC, KP>(safe, o));
+    return ESPM_OK;
 }
 
-// defined in xpass_f32f32.cu / xpass_f32f64.cu / xpass_f64f64.cu
-int xpass_f32f32(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream);
-int xpass_f32f64(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream);
-int xpass_f64f64(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream);
+// The launchers of one (storage, compute) pair; one row per pair is defined in stream_<pair>.cu.
+// fit_stats and w_info with bytes_out != NULL only report the scratch bytes of the launch.
+struct StreamPair {
+    int x_dtype, c_dtype;   // ESPM_F32 / ESPM_F64 / ESPM_U8 / ESPM_U16
+    int (*xpass)(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t s);
+    int (*xpass_sizes)(int kp, int safe, XPassSizes* o);
+    // pixel_out [4][p_loc], channel_out [4][n]
+    int (*fit_stats)(const espm_state* st, double* pixel_out, double* channel_out, void* scratch, int64_t* bytes_out,
+                     cudaStream_t s);
+    // out: [k + 2 k (k + 1) / 2][p_loc] doubles (std rows, packed C, packed F)
+    int (*h_info)(const espm_state* st, int simplex, double* out, cudaStream_t s);
+    // out: [k (k + 1) / 2][n] doubles (packed A_c)
+    int (*w_info)(const espm_state* st, double* out, void* scratch, int64_t* bytes_out, cudaStream_t s);
+};
+extern const StreamPair stream_f32f32, stream_f32f64, stream_f64f64;
 // compact count storage (SURVEY.md section 8f-4): uint8 / uint16 X with fp32 arithmetic
-int xpass_u8f32(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream);
-int xpass_u16f32(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t stream);
+extern const StreamPair stream_u8f32, stream_u16f32;
 
 }  // namespace espm

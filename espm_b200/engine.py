@@ -342,9 +342,7 @@ class FitEngine:
         """Per-pixel and per-channel sums of x, y, kl and chi2 of (W_cur, H_cur) against X (espm_fit_stats): this rank's
         (4, p_loc) pixel block and (4, n) channel block, device float64 tensors."""
         st, dev = self.st, self.device
-        nbytes = ctypes.c_int64(0)
-        L.check(self.lib.espm_fit_stats_scratch(ctypes.byref(st), ctypes.byref(nbytes)))
-        scratch = torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=dev)
+        scratch = self._scratch(self.lib.espm_fit_stats_scratch)
         pix = torch.empty(4, self.p_loc, dtype=torch.float64, device=dev)
         chan = torch.empty(4, self.n, dtype=torch.float64, device=dev)
         L.check(self.lib.espm_fit_stats(ctypes.byref(st), pix.data_ptr(), chan.data_ptr(), scratch.data_ptr(),
@@ -366,15 +364,19 @@ class FitEngine:
         """Poisson information of the phases per channel given H_cur (espm_phase_info): this rank's (k(k+1)/2, n) device
         float64 tensor of A_c[a, b] = sum_j x_cj h_aj h_bj / y_cj^2 as packed upper triangles, row by row."""
         st, dev = self.st, self.device
-        nbytes = ctypes.c_int64(0)
-        L.check(self.lib.espm_phase_info_scratch(ctypes.byref(st), ctypes.byref(nbytes)))
-        scratch = torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=dev)
+        scratch = self._scratch(self.lib.espm_phase_info_scratch)
         out = torch.empty(self.k * (self.k + 1) // 2, self.n, dtype=torch.float64, device=dev)
         L.check(self.lib.espm_phase_info(ctypes.byref(st), out.data_ptr(), scratch.data_ptr(), self.stream))
         self.n_launches += 3                                 # the H tiles, the streaming kernel and the fold of its slots
         return out
 
     # ------------------------------------------------------------------ helpers
+    def _scratch(self, query):
+        """Device scratch of at least the bytes that ``query`` (an espm_*_scratch entry point) reports, and >= 8."""
+        nbytes = ctypes.c_int64(0)
+        L.check(query(ctypes.byref(self.st), ctypes.byref(nbytes)))
+        return torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=self.device)
+
     @property
     def stream(self):
         return ctypes.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)

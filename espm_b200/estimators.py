@@ -612,19 +612,13 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         ``G_`` as fitted.  ``algo``, ``l2`` and the regularisers play no part.  Returns a ``FitStatistics``; the residual
         sum spectrum is ``channel_counts - channel_model``.  Leaves every fitted attribute unchanged.  In a pixel-sharded
         run every rank passes the whole X and gets the whole, identical, result."""
-        import torch
         eng, shard, p = self._statistics_engine(X, H)
         try:
             pix, chan = eng.fit_statistics()
             if shard is None:
                 pix, chan = pix.cpu().numpy(), chan.cpu().numpy()
             else:
-                import torch.distributed as dist
-                parts = [torch.empty_like(chan) for _ in range(shard.world)]
-                dist.all_gather(parts, chan, group=shard.group)
-                for r in range(1, shard.world):               # rank order: the same bits on every rank
-                    parts[0] += parts[r]
-                chan = parts[0].cpu().numpy()
+                chan = self._sum_ranks(shard, chan)
                 pix = self._gather_pixels(eng, shard, p, pix)
         finally:
             eng.close()
@@ -700,19 +694,11 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         spectrum_std; with G = None only that channel (e.g. one without counts), which is then left out of M, as a fixed
         entry is.  ``information`` is always returned.  Nothing is printed and no fitted attribute changes.  In a
         pixel-sharded run every rank passes the whole X and gets the whole, identical, result."""
-        import torch
         from .host import phase_covariance
         eng, shard, _ = self._statistics_engine(X, H)
         try:
             A = eng.phase_information()
-            if shard is not None:
-                import torch.distributed as dist
-                parts = [torch.empty_like(A) for _ in range(shard.world)]
-                dist.all_gather(parts, A, group=shard.group)
-                for r in range(1, shard.world):               # rank order: the same bits on every rank
-                    parts[0] += parts[r]
-                A = parts[0]
-            A = A.cpu().numpy()
+            A = A.cpu().numpy() if shard is None else self._sum_ranks(shard, A)
         finally:
             eng.close()
         m, k = self.W_.shape
@@ -751,6 +737,18 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         eng = FitEngine.for_statistics(Xv, None if self._identity_G else self.G_, self.W_, np.asarray(H),
                                        log_shift=self.log_shift, shard=shard)
         return eng, shard, p
+
+    @staticmethod
+    def _sum_ranks(shard, block):
+        """The host array of the sum over ranks of every rank's device block, added in rank order so that every rank gets
+        the same bits."""
+        import torch
+        import torch.distributed as dist
+        parts = [torch.empty_like(block) for _ in range(shard.world)]
+        dist.all_gather(parts, block, group=shard.group)
+        for r in range(1, shard.world):
+            parts[0] += parts[r]
+        return parts[0].cpu().numpy()
 
     @staticmethod
     def _gather_pixels(eng, shard, p, block):
