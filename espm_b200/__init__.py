@@ -6,8 +6,10 @@ All arithmetic runs in hand-written CUDA kernels (``espm_b200/csrc``) behind the
 ``include/espm_b200.h``; there is no CPU fallback.
 """
 from . import config  # noqa: F401
-from .estimators import AbundanceUncertainty, FitStatistics, PhaseUncertainty, SmoothNMF  # noqa: F401
+from .estimators import (AbundanceUncertainty, FitStatistics, PhaseUncertainty, ResidualComponents,  # noqa: F401
+                         SmoothNMF)
 from . import ops  # noqa: F401
 
-__all__ = ["SmoothNMF", "FitStatistics", "AbundanceUncertainty", "PhaseUncertainty", "ops", "config"]
+__all__ = ["SmoothNMF", "FitStatistics", "AbundanceUncertainty", "PhaseUncertainty", "ResidualComponents", "ops",
+           "config"]
 __version__ = "0.1.0"

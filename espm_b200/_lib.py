@@ -144,6 +144,10 @@ _EXPORTS = {
     "espm_abundance_info": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.c_int, _vp, _vp]),
     "espm_phase_info_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), ctypes.POINTER(_i64)]),
     "espm_phase_info": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _vp, _vp]),
+    "espm_resid_left_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), _i32, ctypes.POINTER(_i64)]),
+    "espm_resid_left": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _i32, _vp, _vp, _vp]),
+    "espm_resid_right_scratch": (ctypes.c_int, [ctypes.POINTER(EspmState), _i32, ctypes.POINTER(_i64)]),
+    "espm_resid_right": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp, _i32, _vp, _vp, _vp]),
     "espm_h_finish": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_h_apply": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),
     "espm_w_pass": (ctypes.c_int, [ctypes.POINTER(EspmState), _vp]),

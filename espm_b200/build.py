@@ -21,7 +21,7 @@ LIBPATH = os.path.join(LIBDIR, LIBNAME)
 SOURCES = ["api.cu", "stream_f32f32.cu", "stream_f32f64.cu", "stream_f64f64.cu", "stream_u8f32.cu", "stream_u16f32.cu",
            "small_f32.cu", "small_f64.cu", "ingest.cu"]
 HEADERS = ["common.cuh", "xpass.cuh", "xpass_inst.cuh", "small.cuh", "small_inst.cuh", "ingest.cuh", "ingest_decl.h",
-           "fitstats.cuh", "hinfo.cuh", "winfo.cuh", os.path.join("..", "..", "include", "espm_b200.h")]
+           "fitstats.cuh", "hinfo.cuh", "winfo.cuh", "resid.cuh", os.path.join("..", "..", "include", "espm_b200.h")]
 
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 NVCC_FLAGS = [

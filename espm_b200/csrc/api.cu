@@ -445,6 +445,56 @@ int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stre
     return stream_pair(st)->w_info(st, out, scratch, nullptr, (cudaStream_t)stream);
 }
 
+static int resid_check(const espm_state* st, int r, const char* what) {
+    int rc = check_state(st);
+    if (rc) return rc;
+    if (r < 1) {
+        set_error("%s: r=%d columns, at least 1 required", what, r);
+        return ESPM_ERR_BAD_ARG;
+    }
+    return ESPM_OK;
+}
+
+int espm_resid_left_scratch(const espm_state* st, int r, int64_t* bytes_out) {
+    int rc = resid_check(st, r, "espm_resid_left_scratch");
+    if (rc) return rc;
+    if (!bytes_out) {
+        set_error("espm_resid_left_scratch: null output");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return stream_pair(st)->resid_left(st, nullptr, r, nullptr, nullptr, bytes_out, nullptr);
+}
+
+int espm_resid_left(const espm_state* st, const double* Q, int r, double* out, void* scratch, void* stream) {
+    int rc = resid_check(st, r, "espm_resid_left");
+    if (rc) return rc;
+    if (!Q || !out || !scratch || !st->Xt || !st->GWc_cur || !st->H_cur) {
+        set_error("espm_resid_left: null input, output or scratch buffer");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return stream_pair(st)->resid_left(st, Q, r, out, scratch, nullptr, (cudaStream_t)stream);
+}
+
+int espm_resid_right_scratch(const espm_state* st, int r, int64_t* bytes_out) {
+    int rc = resid_check(st, r, "espm_resid_right_scratch");
+    if (rc) return rc;
+    if (!bytes_out) {
+        set_error("espm_resid_right_scratch: null output");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return stream_pair(st)->resid_right(st, nullptr, r, nullptr, nullptr, bytes_out, nullptr);
+}
+
+int espm_resid_right(const espm_state* st, const double* P, int r, double* out, void* scratch, void* stream) {
+    int rc = resid_check(st, r, "espm_resid_right");
+    if (rc) return rc;
+    if (!P || !out || !scratch || !st->Xt || !st->GWc_cur || !st->H_cur) {
+        set_error("espm_resid_right: null input, output or scratch buffer");
+        return ESPM_ERR_BAD_ARG;
+    }
+    return stream_pair(st)->resid_right(st, P, r, out, scratch, nullptr, (cudaStream_t)stream);
+}
+
 int espm_w_pass(const espm_state* st, void* stream) {
     int rc = check_state(st);
     if (rc) return rc;

@@ -97,7 +97,7 @@ static int xpass_sizes(int kp, int safe, XPassSizes* o) {
 }
 
 // The launchers of one (storage, compute) pair; one row per pair is defined in stream_<pair>.cu.
-// fit_stats and w_info with bytes_out != NULL only report the scratch bytes of the launch.
+// fit_stats, w_info and the residual products with bytes_out != NULL only report the scratch bytes of the launch.
 struct StreamPair {
     int x_dtype, c_dtype;   // ESPM_F32 / ESPM_F64 / ESPM_U8 / ESPM_U16
     int (*xpass)(const XPassLaunch& l, const XPassArgs* a, int* occ_out, cudaStream_t s);
@@ -109,6 +109,11 @@ struct StreamPair {
     int (*h_info)(const espm_state* st, int simplex, double* out, cudaStream_t s);
     // out: [k (k + 1) / 2][n] doubles (packed A_c)
     int (*w_info)(const espm_state* st, double* out, void* scratch, int64_t* bytes_out, cudaStream_t s);
+    // products of the Pearson residual: left out [r][p_loc] = R^T Q (Q [n][r]), right out [n][r] = R P^T (P [r][p_loc])
+    int (*resid_left)(const espm_state* st, const double* Q, int r, double* out, void* scratch, int64_t* bytes_out,
+                      cudaStream_t s);
+    int (*resid_right)(const espm_state* st, const double* P, int r, double* out, void* scratch, int64_t* bytes_out,
+                       cudaStream_t s);
 };
 extern const StreamPair stream_f32f32, stream_f32f64, stream_f64f64;
 // compact count storage (SURVEY.md section 8f-4): uint8 / uint16 X with fp32 arithmetic

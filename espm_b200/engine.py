@@ -38,6 +38,11 @@ def _torch_dtype(code):
 
 
 _X_ITEMSIZE = {L.F32: 4, L.F64: 8, L.U8: 1, L.U16: 2}
+RESID_RB = 16     # columns per launch of the residual products (RESID_RB of csrc/resid.cuh)
+
+
+def _resid_blocks(r):
+    return -(-r // RESID_RB)
 
 
 def _code_of(dtype):
@@ -370,11 +375,37 @@ class FitEngine:
         self.n_launches += 3                                 # the H tiles, the streaming kernel and the fold of its slots
         return out
 
+    def residual_left(self, Q):
+        """R^T Q of the Pearson residual R = (x - y) / sqrt(y) of (W_cur, H_cur) (espm_resid_left): Q is (n, r), host or
+        device; returns this rank's (r, p_loc) device float64 tensor."""
+        Q = torch.as_tensor(Q, dtype=torch.float64, device=self.device).contiguous()
+        r = Q.shape[1]
+        assert Q.shape == (self.n, r) and r >= 1
+        scratch = self._scratch(self.lib.espm_resid_left_scratch, r)
+        out = torch.empty(r, self.p_loc, dtype=torch.float64, device=self.device)
+        L.check(self.lib.espm_resid_left(ctypes.byref(self.st), Q.data_ptr(), r, out.data_ptr(), scratch.data_ptr(),
+                                         self.stream))
+        self.n_launches += 2 * _resid_blocks(r)              # per block of columns: the [g | Q] rows, the streaming kernel
+        return out
+
+    def residual_right(self, P):
+        """R P^T of the Pearson residual of (W_cur, H_cur) (espm_resid_right): P is this rank's (r, p_loc), host or
+        device; returns this rank's (n, r) device float64 tensor."""
+        P = torch.as_tensor(P, dtype=torch.float64, device=self.device).contiguous()
+        r = P.shape[0]
+        assert P.shape == (r, self.p_loc) and r >= 1
+        scratch = self._scratch(self.lib.espm_resid_right_scratch, r)
+        out = torch.empty(self.n, r, dtype=torch.float64, device=self.device)
+        L.check(self.lib.espm_resid_right(ctypes.byref(self.st), P.data_ptr(), r, out.data_ptr(), scratch.data_ptr(),
+                                          self.stream))
+        self.n_launches += 3 * _resid_blocks(r)              # per block: the [h; P] tiles, the streaming kernel, the fold
+        return out
+
     # ------------------------------------------------------------------ helpers
-    def _scratch(self, query):
+    def _scratch(self, query, *args):
         """Device scratch of at least the bytes that ``query`` (an espm_*_scratch entry point) reports, and >= 8."""
         nbytes = ctypes.c_int64(0)
-        L.check(query(ctypes.byref(self.st), ctypes.byref(nbytes)))
+        L.check(query(ctypes.byref(self.st), *args, ctypes.byref(nbytes)))
         return torch.empty(max(nbytes.value // 8, 1), dtype=torch.float64, device=self.device)
 
     @property

@@ -16,7 +16,9 @@ fitted phases held fixed (only the H half of an iteration runs).  ``goodness_of_
 explains the data and where it does not (per-pixel and per-channel KL and chi-square sums, one pass over X), and
 ``abundance_uncertainty`` how precise the maps are (per-pixel standard errors and covariances from the Poisson
 information, one pass over X), and ``phase_uncertainty`` how precise the phases are (standard errors and covariances of
-``W_`` and error bands of the phase spectra, from the per-channel Poisson information, one pass over X).  Pixel-sharded fits (one process per GPU) support every
+``W_`` and error bands of the phase spectra, from the per-channel Poisson information, one pass over X), and
+``residual_components`` what the model misses (the leading singular triplets of its Pearson residual, by a randomized
+SVD whose products stream X on the device).  Pixel-sharded fits (one process per GPU) support every
 algorithm, loss and option, including ``linesearch`` and ground-truth tracking.
 """
 import sys
@@ -59,6 +61,12 @@ m, k) the covariance and Poisson information of vec(W).  With G = None (m = n): 
 only, ``covariance`` and ``information`` (n, k, k), one per channel.  ``spectrum_std`` (n, k) is the standard error of
 the phase spectra G W (``components_``).  NaN marks singular information: all of std, covariance and spectrum_std with a
 real G, the channel's entries with G = None."""
+
+ResidualComponents = namedtuple("ResidualComponents", ["singular_values", "spectra", "maps"])
+ResidualComponents.__doc__ = """Leading singular triplets of the Pearson residual (x - y) / sqrt(y) of a SmoothNMF model
+(``SmoothNMF.residual_components``), float64 arrays: ``singular_values`` (rank,) descending, ``spectra`` (n, rank) with
+orthonormal columns (the channel side; the entry of largest magnitude of each column is positive) and ``maps`` (rank, p)
+with orthonormal rows (the pixel side, pixel order of the X passed in)."""
 
 
 class SmoothNMF(TransformerMixin, BaseEstimator):
@@ -709,6 +717,84 @@ class SmoothNMF(TransformerMixin, BaseEstimator):
         if self.simplex_W:
             rows = np.arange(m) if self.physics_model_ is None else np.asarray(self.physics_model_.NMF_simplex())
         return PhaseUncertainty(*phase_covariance(A, None if self._identity_G else self.G_, free, rows))
+
+    def residual_components(self, X, rank=4, H=None, n_iter=7, random_state=None):
+        """What the fitted model misses: the leading singular values and vectors of its Pearson residual, by a randomized
+        SVD whose passes over X run on the device.
+
+        With g = max(G_ W_, log_shift), h = max(H, log_shift) and y = g h (the clamped model of the KL loss, as in
+        ``goodness_of_fit``), the residual is R[c, j] = (x_cj - y_cj) / sqrt(y_cj), an (n, p) matrix whose squared
+        Frobenius norm is the total Pearson chi-square of ``goodness_of_fit``.  Where the model is right its entries have
+        unit variance; structure the model lacks (a missing phase, an element line, a detector artefact) shows up as a
+        component with a large singular value, a spectrum with the lines and a map with the shape of what is missing.
+
+        The values are descriptive: there is no built-in significance threshold.  For low-count data the Pearson entries
+        are far from Gaussian, so the Marchenko-Pastur edge sqrt(n) + sqrt(p) is not a reliable noise level.  Compare
+        instead with the same call on a Poisson replicate of the fitted model, e.g.
+        ``est.residual_components(rng.poisson(est.G_ @ est.W_ @ H), rank)``: components that stand well above the
+        replicate's are structure the model misses.
+
+        Algorithm: randomized subspace iteration on the channel side with r = rank + 10 columns (``host.
+        residual_components``); each of the 2 n_iter + 1 products R^T Q / R P^T is one pass over X per 16 columns.
+
+        X : the data, laid out as for ``fit_transform``, with the n channels of the fitted ``G_``.  Used as given; NaN,
+            inf and negative entries raise the errors of ``fit``.
+        rank : number of components, an integer with 1 <= rank <= min(n, p) - 10.
+        H : (k, p) maps in the internal orientation, e.g. ``est.transform(X_b).T`` for a new image; by default the
+            fitted ``H_``.
+        n_iter : power iterations (>= 0).  Each sharpens the separation of the components by another factor
+            (s_i / s_(r+1))^2; with n_iter = 0 the result is R projected on the random start only (values below the
+            true ones).
+        random_state : seed of the Gaussian start (scikit-learn's ``check_random_state``).
+
+        Returns a ``ResidualComponents``: ``singular_values`` (rank,) descending, ``spectra`` (n, rank) with orthonormal
+        columns and ``maps`` (rank, p) with orthonormal rows (reshape a row with ``shape_2d``); in every component the
+        entry of ``spectra[:, i]`` of largest magnitude is positive.  Nothing is printed and no fitted attribute changes.
+        In a pixel-sharded run every rank passes the whole X and gets the whole, identical, result."""
+        import torch
+        from sklearn.utils import check_random_state
+        from .host import RESID_OVERSAMPLE, residual_components
+        check_is_fitted(self, "G_")
+        if isinstance(rank, (bool, np.bool_)) or not isinstance(rank, (int, np.integer)):
+            raise ValueError("rank must be an integer, got %r" % (rank,))
+        if isinstance(n_iter, (bool, np.bool_)) or not isinstance(n_iter, (int, np.integer)) or n_iter < 0:
+            raise ValueError("n_iter must be an integer >= 0, got %r" % (n_iter,))
+        shape = np.shape(X)
+        if len(shape) == 2:
+            n, p = shape[::-1] if self.hspy_comp else shape
+            if not 1 <= rank <= min(n, p) - RESID_OVERSAMPLE:
+                raise ValueError("rank must be between 1 and min(n, p) - %d = %d, got %d"
+                                 % (RESID_OVERSAMPLE, min(n, p) - RESID_OVERSAMPLE, rank))
+        elif rank < 1:
+            raise ValueError("rank must be >= 1, got %d" % rank)
+        rng = check_random_state(random_state)
+        rank, n_iter = int(rank), int(n_iter)
+        r = rank + RESID_OVERSAMPLE
+        Q0 = rng.standard_normal((self.G_.shape[0], r))
+        eng, shard, p = self._statistics_engine(X, H)
+        try:
+            if shard is not None:                            # the start of rank 0, so that an unseeded call agrees too
+                import torch.distributed as dist
+                t = torch.as_tensor(Q0, device=eng.device)
+                dist.broadcast(t, src=shard._peer(0), group=shard.group)
+                Q0 = t.cpu().numpy()
+
+            def right(P):
+                Y = eng.residual_right(P)
+                return Y.cpu().numpy() if shard is None else self._sum_ranks(shard, Y)
+
+            def gram(P):
+                Ph = P.cpu().numpy()
+                M = Ph @ Ph.T
+                return M if shard is None else self._sum_ranks(shard, torch.as_tensor(M, device=eng.device))
+
+            s, spectra, V, P = residual_components(eng.residual_left, right, gram, Q0, rank, n_iter)
+            maps = V.T @ P.cpu().numpy()
+            if shard is not None:
+                maps = self._gather_pixels(eng, shard, p, torch.as_tensor(maps, device=eng.device))
+        finally:
+            eng.close()
+        return ResidualComponents(s, spectra, np.ascontiguousarray(maps))
 
     def _statistics_engine(self, X, H):
         """Checks the arguments of goodness_of_fit / abundance_uncertainty / phase_uncertainty (before any device work)

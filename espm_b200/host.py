@@ -237,3 +237,37 @@ def _block_covariance(A, free, simplex_rows):
     std = np.sqrt(np.maximum(np.diagonal(C, axis1=1, axis2=2), 0.0))
     std[~ok] = np.nan
     return std, C, A, std.copy()
+
+
+RESID_OVERSAMPLE = 10   # extra columns of the residual subspace iteration (scikit-learn's randomized_svd default)
+
+
+def residual_components(left, right, gram, Q0, rank, n_iter):
+    """Leading ``rank`` singular triplets of the residual R (n x p) by randomized subspace iteration on the channel side,
+    in fp64, with R reached only through three callables:
+
+        left(Q)  this rank's P = (R^T Q)^T, (r, p_loc), for an orthonormal Q (n, r) (one pass over X)
+        right(P) R P^T summed over the ranks in rank order, (n, r) host array (one pass over X)
+        gram(P)  P P^T summed over the ranks in rank order, (r, r) host array
+
+    Q0 (n, r) is the Gaussian start, identical on every rank.  Q = qr(Q0); n_iter times Q = qr(R R^T Q); then
+    P = (R^T Q)^T, M = P P^T = U diag(s^2) U^T, spectra = Q U and maps = (P^T U / s)^T.  Every tall factorisation is on
+    the n side (n x r QR); no p x r panel is gathered.  Forming M squares the condition: component i loses about
+    eps (s_1 / s_i)^2 of relative accuracy, harmless in fp64 for the leading components returned.  Sign: the entry of
+    largest magnitude of every spectrum is positive.
+
+    Returns (s (rank,), spectra (n, rank), V (r, rank), P): this rank's maps are V^T P."""
+    Q = np.linalg.qr(np.asarray(Q0, dtype=np.float64))[0]
+    for _ in range(n_iter):
+        Q = np.linalg.qr(right(left(Q)))[0]
+    P = left(Q)
+    w, U = np.linalg.eigh(gram(P))
+    order = np.argsort(w, kind="stable")[::-1][:rank]
+    s = np.sqrt(np.maximum(w[order], 0.0))
+    U = U[:, order]
+    spectra = Q @ U
+    lead = spectra[np.argmax(np.abs(spectra), axis=0), np.arange(rank)]
+    sign = np.where(lead < 0, -1.0, 1.0)
+    spectra *= sign
+    V = U * (sign / np.where(s > 0, s, np.inf))
+    return s, spectra, V, P

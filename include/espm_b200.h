@@ -190,7 +190,7 @@ typedef struct espm_state {
     const void* GW_cur;     /* n_pad x kp */
     const void* GWc_cur;    /* max(GW, ls), n_pad x kp (written by every espm_gw_prepare; read by the X passes only with
                              * ESPM_FLAG_LOSS_DUAL, always by espm_fit_stats,
-                             * espm_abundance_info and espm_phase_info) */
+                             * espm_abundance_info, espm_phase_info and the espm_resid_* products) */
     void* GW_next;
     void* GWc_next;
     void* gwstats_cur;      /* 2*kp (c dtype): colsum(GW), colsum(max(GW,ls)) over the n real rows */
@@ -393,6 +393,22 @@ int espm_abundance_info(const espm_state* st, int simplex, double* out, void* st
  */
 int espm_phase_info_scratch(const espm_state* st, int64_t* bytes_out);
 int espm_phase_info(const espm_state* st, double* out, void* scratch, void* stream);
+/*
+ * Products of the Pearson residual of (GW_cur, H_cur) with a block of vectors, over this rank's pixels
+ * (SmoothNMF.residual_components), one pass over Xt per 16 columns:
+ *   y_cj = sum_a g_ca h_aj,   g = max(GW, ls), h = max(H, ls)       (the clamped Y of the KL loss)
+ *   R_cj = (x_cj - y_cj) / sqrt(y_cj)
+ *   espm_resid_left:  out [r][p_loc] = R^T Q, Q [n][r] (row-major device doubles); H pass order
+ *   espm_resid_right: out [n][r]     = R P^T, P [r][p_loc] (row-major device doubles); W pass order
+ * scratch: espm_resid_left_scratch / espm_resid_right_scratch bytes for the same r (the left product's [g | Q] rows;
+ * the right product's tile-major [h; P] blocks and per-CTA channel sums).
+ * Reads Xt, GWc_cur, H_cur (k x ldh) and log_shift; writes no record and no device flag.  No atomics, fixed summation
+ * order: two calls give identical bits, and a pixel's left product does not depend on the grid or on the sharding.
+ */
+int espm_resid_left_scratch(const espm_state* st, int r, int64_t* bytes_out);
+int espm_resid_left(const espm_state* st, const double* Q, int r, double* out, void* scratch, void* stream);
+int espm_resid_right_scratch(const espm_state* st, int r, int64_t* bytes_out);
+int espm_resid_right(const espm_state* st, const double* P, int r, double* out, void* scratch, void* stream);
 /*
  * Per-pixel assembly (updates.py:132-142): num, den with the log and Laplacian surrogates, the loss
  * regularisers of the CURRENT iterate (measures.py:548,577), rel_H (base.py:324), and either
